@@ -11,6 +11,10 @@ GPU on synthetic 200 Hz IMU + 25 Hz marker poses; one bench "step" = one second 
 periodic in that second, so every step replays the same device-resident noisy streams with timestamps advanced by
 one period: the filters keep running, nothing is reset or cached between steps.
 
+--dump-outputs DIR writes, after the timed steps, what the timed path left its caller: the state of a fixed, seeded sample
+of rank 0's filters and the statistics vector of the whole batch, as float64 DIR/<name>.npy (about 24 MB).  The inputs
+depend only on the arguments, so two builds run with the same arguments can be compared output for output.
+
 One JSON line on stdout (rank 0).  `value` = device-resident inputs; `e2e` = the same call with HOST (pinned)
 buffers, i.e. host->device copies of every step's streams and a device->host read of the step's statistics inside
 the timed region.  The host IMU stream of `e2e` is in the format the reference system receives it in -- the IMSEE SDK's
@@ -29,6 +33,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "oracle")):
     if _p not in sys.path:
@@ -43,6 +48,7 @@ FLOP_SOLVE = 1900.0
 BYTES_SOLVE = 124.0
 PERIOD = 1.0  # seconds of stream per bench step
 IMU_RATE, FRAME_RATE = 200.0, 25.0
+DUMP_FILTERS = 8192  # filters whose whole state --dump-outputs writes: 363 doubles each, ~24 MB
 
 
 def env_int(name, default):
@@ -235,6 +241,14 @@ def run_ours(args):
 
     B = env_int("FBUS_BENCH_BATCH", 1 << 20)
     K, Wm = args.steps, args.warmup
+    if args.dump_outputs and rank == 0:
+        # fbus_get_state reads the whole batch: host copy of every field + the library's staging of the packed covariance
+        import psutil
+        need = B * 8 * (sum(n for _, n, _ in capi.STATE_FIELDS) + 18 * 19 // 2)
+        avail = psutil.virtual_memory().available
+        if need > 0.8 * avail:
+            raise SystemExit(f"bench.py: --dump-outputs reads the state of all {B} filters, {need / 1e9:.1f} GB of host memory; "
+                             f"{avail / 1e9:.1f} GB are available")
     cfg = capi.config_default()
     traj = synth.truth_trajectory(cfg, PERIOD, IMU_RATE, FRAME_RATE, periodic=True)
     N, W = traj["base_imu"].shape[0], traj["base_pose"].shape[0]
@@ -293,8 +307,11 @@ def run_ours(args):
     f.Synchronize()
     from fbus_ekf_b200 import shard
     shard.combine_stats(st_d, dist if world > 1 else None)  # SUM of the sums, MAX of the maximum
-    stats = shard.summarize_stats(st_d.cpu().numpy())
+    stats_vec = st_d.cpu().numpy()
+    stats = shard.summarize_stats(stats_vec)
     stats.update({"after_seconds_of_stream": (k_last + 1) * PERIOD, "allreduce": "nccl" if world > 1 else "single rank"})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, f, stats_vec)  # before the e2e_montecarlo leg steps `f` further
 
     # ---- roofline of the dominant kernel (ekf_window_kernel) -------------------------------------------------------
     flop_launch = B * (N * FLOP_IMU_STEP + W * FLOP_UPDATE)
@@ -777,6 +794,23 @@ def bench_strong(cfg, traj, local, rank, dev, world, K, Wm, weak_value):
                     "filters per GPU; CUDA events on each rank's stream, barrier both sides, max over ranks"}
 
 
+def dump_outputs(out_dir, f, stats_vec):
+    """--dump-outputs: the state fbus_get_state returns after the last timed step (every field, covariance included) for
+    DUMP_FILTERS filters (FBUS_BENCH_DUMP_FILTERS) drawn with a fixed seed (all of them for a smaller batch), their indices,
+    and the statistics vector of the whole batch; all as float64 .npy files."""
+    n = env_int("FBUS_BENCH_DUMP_FILTERS", DUMP_FILTERS)
+    st = f.GetState()
+    if f.batch <= n:
+        idx = np.arange(f.batch)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(f.batch, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "filter_index.npy"), idx.astype(np.float64))
+    for name, a in st.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a[..., idx], dtype=np.float64))
+    np.save(os.path.join(out_dir, "stats.npy"), np.asarray(stats_vec, dtype=np.float64))
+
+
 def library_build_info():
     """which build of the CUDA library ran: its source hash, and whether this process compiled it or found it prebuilt"""
     try:
@@ -804,7 +838,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-solves", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state after the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm times bounded CPU samples")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

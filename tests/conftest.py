@@ -33,7 +33,9 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(ROOT, "tests", "golden", "fbus_logs.npz"))
+    """the reference's bundled logs, {"land_imu": rows, ...}, from tests/golden/*.txt.xz (see make_golden.py)"""
+    return {f"{log}_{kind}": np.loadtxt(os.path.join(ROOT, "tests", "golden", f"{log}_{kind}.txt.xz"), ndmin=2)
+            for log in ("land", "water") for kind in ("corners", "image", "imu", "fusion")}
 
 
 @pytest.fixture(scope="session")
