@@ -27,6 +27,9 @@ FBUS_FLAG_JOSEPH = 0x1
 FBUS_FLAG_MATLAB = 0x2
 FBUS_MAX_MARKERS = 16
 FBUS_NSTATS = 8
+# rows of a per-filter noise array (fbus_set_noise), in fbus_config order
+NOISE_FIELDS = ("accel_n_cov", "gyro_n_cov", "accel_b_cov", "gyro_b_cov", "pos_n_cov", "quat_n_cov")
+FBUS_NOISE_FIELDS = len(NOISE_FIELDS)
 
 ST_INIT_FAILED = 0x1
 ST_RESET_SKIPPED = 0x2
@@ -167,6 +170,8 @@ def lib() -> C.CDLL:
         "fbus_clear_status": (C.c_int, [H]),
         "fbus_stats": (C.c_int, [H, C.c_void_p, C.c_void_p, C.c_int32, c_double_p, C.c_void_p]),
         "fbus_stats_combine": (C.c_int, [c_double_p, C.c_size_t, c_double_p]),
+        "fbus_set_noise": (C.c_int, [H, C.c_void_p, C.c_int32]),
+        "fbus_filter_errors": (C.c_int, [H, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]),
         "fbus_stats_allreduce": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p), c_double_p]),
         "fbus_stats_allreduce_comm": (C.c_int, [H, C.c_void_p, C.c_void_p, c_double_p]),
         "fbus_synth_streams": (C.c_int, [H, C.POINTER(SynthSpec), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -189,7 +194,7 @@ EXPORTED_SYMBOLS = (
     "fbus_batch", "fbus_stream", "fbus_init_gravity_gyrobias", "fbus_iir_prefilter", "fbus_init_position_quaternion", "fbus_propagate",
     "fbus_reset_state", "fbus_update", "fbus_step_windows", "fbus_refract_solve", "fbus_inair_solve", "fbus_undistort_fisheye", "fbus_solve_to_detections", "fbus_refract_solve_gn", "fbus_marker_pose", "fbus_get_state",
     "fbus_set_state", "fbus_clear_status", "fbus_stats", "fbus_stats_combine", "fbus_stats_allreduce", "fbus_stats_allreduce_comm", "fbus_synth_streams", "fbus_quat_from_rotmat",
-    "fbus_measure_fp64_peak")
+    "fbus_measure_fp64_peak", "fbus_set_noise", "fbus_filter_errors")
 
 
 def config_default() -> FbusConfig:
@@ -206,6 +211,12 @@ def config_matlab() -> FbusConfig:
     if lib().fbus_config_matlab(C.byref(cfg)) != 0:
         raise RuntimeError("fbus_config_matlab failed")
     return cfg
+
+
+def noise_from_config(cfg: FbusConfig, batch: int) -> np.ndarray:
+    """float64 [FBUS_NOISE_FIELDS][batch] array (fbus_set_noise layout) giving every filter the config's values"""
+    col = np.array([getattr(cfg, name) for name in NOISE_FIELDS], dtype=np.float64)
+    return np.ascontiguousarray(np.repeat(col[:, None], int(batch), axis=1))
 
 
 def dptr(a: np.ndarray, typ=c_double_p):

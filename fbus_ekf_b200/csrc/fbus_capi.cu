@@ -82,6 +82,10 @@ struct fbus_handle {
     int32_t* d_init = nullptr;
     int32_t* d_status = nullptr;
     DevBuf imu_t, det_t, win_off, imu_data, det_id, det_pose, trace, scratch_in, scratch_out, scratch_aux, stats_partial, stats_out;
+    DevBuf noise;             // [6][B] per-filter noise values of fbus_set_noise (FBUS_NOISE_FIELDS rows, fbus_config order)
+    bool noise_on = false;    // the window kernels read `noise` instead of the config's values
+    bool noise_smem_set = false;  // shared-memory limits of the NOISE instantiations set (on the first fbus_set_noise)
+    DevBuf errors;            // [4][B] device result of fbus_filter_errors for a host output
     // second staging set + copy stream: host-resident streams are copied chunk c+1 while chunk c is computed
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
@@ -154,7 +158,10 @@ inline void forget_stream_position(fbus_handle* h) {
     h->last_w1 = 0;
 }
 
-int launch_window(fbus_handle* h, WinParams& prm) {
+// NOISE: the instantiations that take every filter's noise values from h->noise (fbus_set_noise); the others get a null
+// pointer they never read
+template <bool NOISE>
+int launch_window_t(fbus_handle* h, WinParams& prm) {
     prm.nom = h->d_nom;
     prm.P = h->d_P;
     prm.prev_id = h->d_prev;
@@ -167,42 +174,73 @@ int launch_window(fbus_handle* h, WinParams& prm) {
     prm.stagger_cycles = (prm.mode & M_FUSED) ? h->stagger_cycles : 0u;
     const unsigned grid = (unsigned)((h->B + WIN_BS - 1) / WIN_BS);
     const bool jo = (h->k.flags & FBUS_FLAG_JOSEPH) != 0, f32 = prm.imu32 != nullptr;
+    const double* const nz = NOISE ? (const double*)h->noise.p : nullptr;
     if (h->k.flags & FBUS_FLAG_MATLAB) {  // MATLAB-semantics mode: the lanes-per-filter kernel at any batch size
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
-        if (f32) ekf_window_lane_kernel<false, true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
-        else ekf_window_lane_kernel<false, false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
+        if (f32) ekf_window_lane_kernel<false, true, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        else ekf_window_lane_kernel<false, false, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
     } else if (h->lane_batch && h->lane_gen == 2) {
         prm.lane_fpc = h->lane_fpc;
         const unsigned g32 = (unsigned)((h->B + h->lane_fpc - 1) / h->lane_fpc);
         if (f32) {
-            if (jo) ekf_window_lane2_kernel<true, true><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k);
-            else ekf_window_lane2_kernel<false, true><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k);
-        } else if (jo) ekf_window_lane2_kernel<true, false><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k);
-        else ekf_window_lane2_kernel<false, false><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k);
+            if (jo) ekf_window_lane2_kernel<true, true, NOISE><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k, nz);
+            else ekf_window_lane2_kernel<false, true, NOISE><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k, nz);
+        } else if (jo) ekf_window_lane2_kernel<true, false, NOISE><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k, nz);
+        else ekf_window_lane2_kernel<false, false, NOISE><<<g32, LANE_NT, LANE2_SMEM, h->stream>>>(prm, h->k, nz);
     } else if (h->lane_batch) {
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
         if (f32) {
-            if (jo) ekf_window_lane_kernel<true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
-            else ekf_window_lane_kernel<false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
-        } else if (jo) ekf_window_lane_kernel<true, false><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
-        else ekf_window_lane_kernel<false, false><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k);
+            if (jo) ekf_window_lane_kernel<true, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+            else ekf_window_lane_kernel<false, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        else ekf_window_lane_kernel<false, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
     } else if (h->small_batch) {
         // fewer 128-filter CTAs than SMs (e.g. BASELINE configs[2], 4 096 filters): 32-filter CTAs (one covariance + one
         // nominal warp) spread the batch over four times as many SMs
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
         const size_t smem32 = (size_t)(NPK + XCH) * 32 * sizeof(double);
         if (f32) {
-            if (jo) ekf_window_split_kernel<32, true, true><<<g32, 64, smem32, h->stream>>>(prm, h->k);
-            else ekf_window_split_kernel<32, false, true><<<g32, 64, smem32, h->stream>>>(prm, h->k);
-        } else if (jo) ekf_window_split_kernel<32, true><<<g32, 64, smem32, h->stream>>>(prm, h->k);
-        else ekf_window_split_kernel<32, false><<<g32, 64, smem32, h->stream>>>(prm, h->k);
+            if (jo) ekf_window_split_kernel<32, true, true, NOISE><<<g32, 64, smem32, h->stream>>>(prm, h->k, nz);
+            else ekf_window_split_kernel<32, false, true, NOISE><<<g32, 64, smem32, h->stream>>>(prm, h->k, nz);
+        } else if (jo) ekf_window_split_kernel<32, true, false, NOISE><<<g32, 64, smem32, h->stream>>>(prm, h->k, nz);
+        else ekf_window_split_kernel<32, false, false, NOISE><<<g32, 64, smem32, h->stream>>>(prm, h->k, nz);
     } else if (f32) {
-        if (jo) ekf_window_split_kernel<WIN_BS, true, true><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k);
-        else ekf_window_split_kernel<WIN_BS, false, true><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k);
-    } else if (jo) ekf_window_split_kernel<WIN_BS, true><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k);
-    else ekf_window_split_kernel<WIN_BS, false><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k);
+        if (jo) ekf_window_split_kernel<WIN_BS, true, true, NOISE><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k, nz);
+        else ekf_window_split_kernel<WIN_BS, false, true, NOISE><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k, nz);
+    } else if (jo) ekf_window_split_kernel<WIN_BS, true, false, NOISE><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k, nz);
+    else ekf_window_split_kernel<WIN_BS, false, false, NOISE><<<grid, 2 * WIN_BS, WIN_SMEM, h->stream>>>(prm, h->k, nz);
     CUDA_TRY(h, cudaGetLastError());
     return FBUS_OK;
+}
+int launch_window(fbus_handle* h, WinParams& prm) { return h->noise_on ? launch_window_t<true>(h, prm) : launch_window_t<false>(h, prm); }
+
+// the largest dynamic shared memory of every window kernel of one NOISE flavour (the default is 48 KB)
+template <bool NOISE>
+cudaError_t set_window_smem_limits() {
+    const int smem32 = (int)((NPK + XCH) * 32 * sizeof(double));
+    cudaError_t e = cudaSuccess;
+    auto set = [&](const void* fn, size_t bytes) {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    };
+    set((const void*)ekf_window_split_kernel<WIN_BS, false, false, NOISE>, WIN_SMEM);
+    set((const void*)ekf_window_split_kernel<WIN_BS, true, false, NOISE>, WIN_SMEM);
+    set((const void*)ekf_window_split_kernel<WIN_BS, false, true, NOISE>, WIN_SMEM);
+    set((const void*)ekf_window_split_kernel<WIN_BS, true, true, NOISE>, WIN_SMEM);
+    set((const void*)ekf_window_split_kernel<32, false, false, NOISE>, smem32);
+    set((const void*)ekf_window_split_kernel<32, true, false, NOISE>, smem32);
+    set((const void*)ekf_window_split_kernel<32, false, true, NOISE>, smem32);
+    set((const void*)ekf_window_split_kernel<32, true, true, NOISE>, smem32);
+    set((const void*)ekf_window_lane_kernel<false, false, false, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<true, false, false, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<false, true, false, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<true, true, false, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<false, false, true, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<false, true, true, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane2_kernel<false, false, NOISE>, LANE2_SMEM);
+    set((const void*)ekf_window_lane2_kernel<true, false, NOISE>, LANE2_SMEM);
+    set((const void*)ekf_window_lane2_kernel<false, true, NOISE>, LANE2_SMEM);
+    set((const void*)ekf_window_lane2_kernel<true, true, NOISE>, LANE2_SMEM);
+    return e;
 }
 
 int stage_det(fbus_handle* h, const fbus_det_frames* det, size_t w0, size_t w1, WinParams& prm, cudaStream_t big_stream = nullptr) {
@@ -317,11 +355,7 @@ int fbus_create(fbus_handle** out, const fbus_config* cfg, int device, size_t ba
     }
     if ((e = cudaMalloc(&h->d_tab, sizeof(MarkerTable))) != cudaSuccess) return bail("cudaMalloc marker table", e);
     if ((e = cudaMemcpy(h->d_tab, &h->tab, sizeof(MarkerTable), cudaMemcpyHostToDevice)) != cudaSuccess) return bail("marker table copy", e);
-    e = cudaFuncSetAttribute(ekf_window_split_kernel<WIN_BS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<WIN_BS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<WIN_BS, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<WIN_BS, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM);
-    if (e != cudaSuccess) return bail("cudaFuncSetAttribute", e);
+    if ((e = set_window_smem_limits<false>()) != cudaSuccess) return bail("cudaFuncSetAttribute", e);
     {
         cudaDeviceProp prop;
         if ((e = cudaGetDeviceProperties(&prop, device)) != cudaSuccess) return bail("cudaGetDeviceProperties", e);
@@ -345,25 +379,7 @@ int fbus_create(fbus_handle** out, const fbus_config* cfg, int device, size_t ba
             const int v = atoi(fp);
             if (v >= 1 && v <= 32) h->lane_fpc = (uint32_t)v;
         }
-        e = cudaFuncSetAttribute(ekf_window_lane_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
-        if (e != cudaSuccess) return bail("cudaFuncSetAttribute(lane)", e);
         if (const char* lg = getenv("FBUS_LANE_GEN")) h->lane_gen = atoi(lg);
-        e = cudaFuncSetAttribute(ekf_window_lane2_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE2_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE2_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE2_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_lane2_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE2_SMEM);
-        if (e != cudaSuccess) return bail("cudaFuncSetAttribute(lane2)", e);
-        const int smem32 = (int)((NPK + XCH) * 32 * sizeof(double));
-        e = cudaFuncSetAttribute(ekf_window_split_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ekf_window_split_kernel<32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32);
-        if (e != cudaSuccess) return bail("cudaFuncSetAttribute(32)", e);
     }
     if (getenv("FBUS_DEBUG")) {
         int nb = -1;
@@ -393,7 +409,7 @@ int fbus_destroy(fbus_handle* h) {
         if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]);
     }
     DevBuf* bufs[] = {&h->imu_t, &h->det_t, &h->win_off, &h->imu_data, &h->det_id, &h->det_pose, &h->trace,
-                      &h->scratch_in, &h->scratch_out, &h->scratch_aux, &h->stats_partial, &h->stats_out};
+                      &h->scratch_in, &h->scratch_out, &h->scratch_aux, &h->stats_partial, &h->stats_out, &h->noise, &h->errors};
     for (DevBuf* b : bufs) b->release();
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -923,6 +939,52 @@ int fbus_stats(fbus_handle* h, const double* truth_p, const double* truth_q, int
     CUDA_TRY(h, cudaGetLastError());
     if (out_host) {
         CUDA_TRY(h, cudaMemcpyAsync(out_host, dout, FBUS_NSTATS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    }
+    return FBUS_OK;
+}
+
+int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem) {
+    if (!h || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE)) return fail(h, FBUS_E_BADARG, "fbus_set_noise: bad argument");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    if (!noise) {  // back to the config's values and the default kernels; the buffer is kept for a later call
+        h->noise_on = false;
+        return FBUS_OK;
+    }
+    if (!h->noise_smem_set) {  // the NOISE instantiations are prepared when first needed: creation only touches the default ones
+        CUDA_TRY(h, set_window_smem_limits<true>());
+        h->noise_smem_set = true;
+    }
+    const size_t bytes = (size_t)FBUS_NOISE_FIELDS * h->B * sizeof(double);
+    CUDA_TRY(h, h->noise.reserve(bytes));  // allocated on the first call (the size is fixed by the batch)
+    // stream-ordered: kernels enqueued before this call still read the previous values
+    CUDA_TRY(h, cudaMemcpyAsync(h->noise.p, noise, bytes, mem == FBUS_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
+                                h->stream));
+    h->noise_on = true;
+    return FBUS_OK;
+}
+
+int fbus_filter_errors(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem, double* out, int32_t out_mem) {
+    if (!h || !truth_p || !truth_q || !out || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE) ||
+        (out_mem != FBUS_MEM_HOST && out_mem != FBUS_MEM_DEVICE))
+        return fail(h, FBUS_E_BADARG, "fbus_filter_errors: bad argument");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    const size_t B = h->B;
+    const double* tp;
+    const double* tq;
+    int rc = stage(h, h->scratch_in, truth_p, 3 * B, mem, &tp);
+    if (rc) return rc;
+    rc = stage(h, h->scratch_out, truth_q, 4 * B, mem, &tq);
+    if (rc) return rc;
+    double* dout = out;
+    if (out_mem == FBUS_MEM_HOST) {
+        CUDA_TRY(h, h->errors.reserve(4 * B * sizeof(double)));
+        dout = (double*)h->errors.p;
+    }
+    filter_errors_kernel<<<(unsigned)((B + STATS_BS - 1) / STATS_BS), STATS_BS, 0, h->stream>>>(h->d_nom, h->d_P, B, tp, tq, dout);
+    CUDA_TRY(h, cudaGetLastError());
+    if (out_mem == FBUS_MEM_HOST) {
+        CUDA_TRY(h, cudaMemcpyAsync(out, dout, 4 * B * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     }
     return FBUS_OK;

@@ -137,9 +137,10 @@ __device__ __forceinline__ void lane_apply_Fu1(double* x, const double* A, const
 }
 
 // COVARIANCE lanes: warp cw (0..10) holds filters 3cw .. 3cw+2 of the CTA, lane = 9*g + l
-template <bool JOSEPH>
+// NOISE: q0, q1 come from this filter's row of the [6][B] buffer `noise` (fbus_set_noise) instead of k.Qd
+template <bool JOSEPH, bool NOISE = false>
 __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh, int32_t (*sflag)[32],
-                                              int cw, int lane) {
+                                              int cw, int lane, const double* noise = nullptr) {
     constexpr int NT = LANE_NT;
     const size_t B = prm.B;
     const int g = lane / 9, l = lane - 9 * g;
@@ -162,8 +163,12 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
     }
     // process noise on the own diagonal entries (GammaQGamma^T is diagonal, filter.hpp:108-125): column l gets it in row l,
     // column l+9 in row l+9
-    const double q0 = (l >= 3 && l < 6) ? k.Qd[0] : (l >= 6 ? k.Qd[1] : 0.0);
-    const double q1 = (l < 3) ? k.Qd[2] : (l < 6 ? k.Qd[3] : 0.0);
+    double q0 = (l >= 3 && l < 6) ? k.Qd[0] : (l >= 6 ? k.Qd[1] : 0.0);
+    double q1 = (l < 3) ? k.Qd[2] : (l < 6 ? k.Qd[3] : 0.0);
+    if constexpr (NOISE) {  // this filter's own values
+        q0 = (l >= 3 && l < 6) ? noise[b] : (l >= 6 ? noise[B + b] : 0.0);
+        q1 = (l < 3) ? noise[2 * B + b] : (l < 6 ? noise[3 * B + b] : 0.0);
+    }
     for (uint32_t w = prm.w0; w < prm.w1; ++w) {
         cta_bar<NT>();  // (a) the nominal warp has posted the IMU range
         const int fp = (int)((w - prm.w0) & 1u);
@@ -299,18 +304,25 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
     }
 }
 
-template <bool JOSEPH, bool IMU32, bool MATLAB = false>
-__global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k) {
+// NOISE: every filter has its own noise values, `noise` is the [6][B] buffer of fbus_set_noise (the other instantiations never
+// read the parameter)
+template <bool JOSEPH, bool IMU32, bool MATLAB = false, bool NOISE = false>
+__global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k,
+                                                                     const double* __restrict__ noise) {
     extern __shared__ double smem[];
     __shared__ SplitShared sh;
     __shared__ int32_t sflag[3][32];
     const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (wi < 11) {
-        lane_cov_role<JOSEPH>(prm, k, smem, sh, sflag, wi, lane);
+        if constexpr (NOISE) lane_cov_role<JOSEPH, true>(prm, k, smem, sh, sflag, wi, lane, noise);
+        else lane_cov_role<JOSEPH>(prm, k, smem, sh, sflag, wi, lane);
     } else {
         const size_t b0 = (size_t)blockIdx.x * 32 + lane;
         const bool live = b0 < prm.B;
-        nominal_role<32, false, IMU32, true, JOSEPH, MATLAB>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live);
+        if constexpr (NOISE)
+            nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live, nullptr,
+                                                                              nullptr, nullptr, noise);
+        else nominal_role<32, false, IMU32, true, JOSEPH, MATLAB>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live);
     }
 }
 
@@ -330,9 +342,9 @@ __global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __gri
 // ------------------------------------------------------------------------------------------------------------------
 constexpr size_t LANE2_SMEM = (size_t)(L2_TOTAL * 32 + L2_RING + LANE_T * 32) * sizeof(double);
 
-template <bool JOSEPH, bool IMU32>
+template <bool JOSEPH, bool IMU32, bool NOISE = false>  // NOISE: as lane_cov_role
 __device__ __forceinline__ void lane2_cov_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh, int32_t (*sflag)[32],
-                                               Lane2Shared& l2, int cw, int lane) {
+                                               Lane2Shared& l2, int cw, int lane, const double* noise = nullptr) {
     constexpr int NT = LANE_NT;
     const size_t B = prm.B;
     const int g = lane / 9, l = lane - 9 * g;
@@ -357,8 +369,12 @@ __device__ __forceinline__ void lane2_cov_role(const WinParams& prm, const DevCo
         c0[i] = prm.P[(size_t)(a0 * NX - (a0 * (a0 - 1)) / 2 + (b0i - a0)) * B + b];
         c1[i] = prm.P[(size_t)(a1 * NX - (a1 * (a1 - 1)) / 2 + (b1i - a1)) * B + b];
     }
-    const double q0 = (l >= 3 && l < 6) ? k.Qd[0] : (l >= 6 ? k.Qd[1] : 0.0);
-    const double q1 = (l < 3) ? k.Qd[2] : (l < 6 ? k.Qd[3] : 0.0);
+    double q0 = (l >= 3 && l < 6) ? k.Qd[0] : (l >= 6 ? k.Qd[1] : 0.0);
+    double q1 = (l < 3) ? k.Qd[2] : (l < 6 ? k.Qd[3] : 0.0);
+    if constexpr (NOISE) {  // this filter's own values
+        q0 = (l >= 3 && l < 6) ? noise[b] : (l >= 6 ? noise[B + b] : 0.0);
+        q1 = (l < 3) ? noise[2 * B + b] : (l < 6 ? noise[3 * B + b] : 0.0);
+    }
     // the sample this warp's slot will most likely hold in the NEXT chunk (the one right behind the current chunk), loaded a whole
     // chunk of covariance steps (and an update) ahead of its use
     const uint32_t imu_end = (prm.mode & M_FUSED) ? prm.win_off[prm.w1] : prm.prop_first + prm.prop_count;
@@ -543,8 +559,9 @@ __device__ __forceinline__ void lane2_cov_role(const WinParams& prm, const DevCo
     }
 }
 
-template <bool JOSEPH, bool IMU32>
-__global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane2_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k) {
+template <bool JOSEPH, bool IMU32, bool NOISE = false>  // NOISE: as ekf_window_lane_kernel
+__global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane2_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k,
+                                                                      const double* __restrict__ noise) {
     extern __shared__ double smem[];
     __shared__ SplitShared sh;
     __shared__ int32_t sflag[3][32];
@@ -559,14 +576,18 @@ __global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane2_kernel(const __gr
         __syncthreads();
     }
     if (wi < 11) {
-        lane2_cov_role<JOSEPH, IMU32>(prm, k, smem, sh, sflag, l2, wi, lane);
+        if constexpr (NOISE) lane2_cov_role<JOSEPH, IMU32, true>(prm, k, smem, sh, sflag, l2, wi, lane, noise);
+        else lane2_cov_role<JOSEPH, IMU32>(prm, k, smem, sh, sflag, l2, wi, lane);
     } else {
         // a CTA serves lane_fpc filters (<= 32): batches that cannot fill the GPU are spread thin, because a filter-step is the
         // faster the fewer filters share the CTA's nominal warp, schedulers and shared-memory bandwidth
         const size_t b0 = (size_t)blockIdx.x * prm.lane_fpc + lane;
         const bool live = lane < (int)prm.lane_fpc && b0 < prm.B;
-        nominal_role<32, false, IMU32, true, JOSEPH, false, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live, &l2, &s_tab,
-                                                                  smem + (size_t)L2_TOTAL * 32);
+        if constexpr (NOISE)
+            nominal_role<32, false, IMU32, true, JOSEPH, false, true, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live, &l2,
+                                                                            &s_tab, smem + (size_t)L2_TOTAL * 32, noise);
+        else nominal_role<32, false, IMU32, true, JOSEPH, false, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live, &l2, &s_tab,
+                                                                       smem + (size_t)L2_TOTAL * 32);
     }
 }
 

@@ -125,9 +125,18 @@ __device__ __forceinline__ int pair_any(const SplitShared& sh, int wq) { return 
 // ------------------------------------------------------------------------------------------------------------------
 // COVARIANCE role: owns P (shared memory; top-left 9x9 in registers while propagating)
 // ------------------------------------------------------------------------------------------------------------------
-template <int BSF, bool JOSEPH, bool TM>
+// Where the covariance warp of a NOISE instantiation keeps its filters' four process noise values: in shared memory (4 x BSF
+// doubles next to the exchange area) when that still fits the 227 KB a CTA may have.  The 128-filter CTAs with the covariance in
+// shared memory (FBUS_TMEM=0) already take 225 KB; they read the values from the noise buffer through the L1 cache per sample.
+template <int BSF, bool TM>
+constexpr bool noise_q_in_smem = (size_t)((TM ? 0 : NPK) + XCH + 4) * BSF * sizeof(double) + 2048 <= (size_t)227 * 1024;
+
+// NOISE: the filters have their own noise values (fbus_set_noise): `noise` is the [6][B] buffer, `sq` this filter's four process
+// noise values in shared memory (entry stride BSF; nullptr when noise_q_in_smem is false), read where Qv is built instead of being
+// held in registers across the step loop
+template <int BSF, bool JOSEPH, bool TM, bool NOISE = false>
 __device__ __forceinline__ void cov_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh, int32_t (*sflag)[BSF],
-                                         int fl, size_t b, bool live, uint32_t tm_base) {
+                                         int fl, size_t b, bool live, uint32_t tm_base, const double* noise = nullptr, double* sq = nullptr) {
     constexpr int NT = 2 * BSF, NW = BSF / 32;
     constexpr int NPS = TM ? 0 : NPK;  // doubles of P per filter in shared memory
     const size_t B = prm.B;
@@ -141,6 +150,10 @@ __device__ __forceinline__ void cov_role(const WinParams& prm, const DevConsts& 
     else P.s = smem + fl;
     double* const X = smem + (size_t)NPS * BSF + fl;
     const int wq = fl >> 5;
+    if constexpr (NOISE && noise_q_in_smem<BSF, TM>) {  // written and read by this thread only
+#pragma unroll
+        for (int c = 0; c < 4; ++c) sq[(size_t)c * BSF] = noise[(size_t)c * B + b];
+    }
     if constexpr (TM) {
         FBUS_UNROLL
         for (int bj = 0; bj < 6; ++bj)
@@ -182,6 +195,13 @@ __device__ __forceinline__ void cov_role(const WinParams& prm, const DevConsts& 
                     const double u0 = rec[(size_t)18 * BSF], u1 = rec[(size_t)19 * BSF], u2 = rec[(size_t)20 * BSF];
                     const double dt = rec[(size_t)21 * BSF];
                     double Qv[4] = {k.Qd[0], k.Qd[1], k.Qd[2], k.Qd[3]};
+                    if constexpr (NOISE && noise_q_in_smem<BSF, TM>) {
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) Qv[c] = sq[(size_t)c * BSF];
+                    } else if constexpr (NOISE) {
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) Qv[c] = __ldg(noise + (size_t)c * B + b);
+                    }
                     if (TM && !valid) Qv[0] = Qv[1] = Qv[2] = Qv[3] = 0.0;  // the record of an invalid sample is all zeros
                     P.fence_st();  // the previous step's stores
                     propagate_cov_core<BSF, true>(P, A, Bm, u0, u1, u2, dt, Qv, TL);
@@ -208,7 +228,12 @@ __device__ __forceinline__ void cov_role(const WinParams& prm, const DevConsts& 
                 t.t = 0.0;
                 const MarkerConst mkc = prm.tab->mk[(req > 0 ? req : 1) - 1];
                 P.fence_st();
-                measurement_update<BSF, JOSEPH ? 1 : 0, BSF>(P, t, k, mkc, yP, yQ, X, req != 0);
+                if constexpr (NOISE) {  // R of this filter, read at the update
+                    const MeasNoise r{noise[4 * B + b], noise[5 * B + b]};
+                    measurement_update<BSF, JOSEPH ? 1 : 0, BSF>(P, t, k, r, mkc, yP, yQ, X, req != 0);
+                } else {
+                    measurement_update<BSF, JOSEPH ? 1 : 0, BSF>(P, t, k, mkc, yP, yQ, X, req != 0);
+                }
                 P.fence_st();
                 // hand back: corrected p, q and the increments of v, b_a, b_g, g
 #pragma unroll
@@ -566,15 +591,18 @@ struct P6View {
 // records need no neutral content, and the update is split differently -- this warp (one lane per filter) runs the
 // state-only prologue (predicted measurement, Hs, S, the gain factors) from the published P6 and the error-state
 // injection, the covariance lanes run the sweep P -= Z^T Z and dx = Z^T y.
-template <int BSF, bool TM, bool IMU32 = false, bool LANE = false, bool JOSEPH = false, bool MATLAB = false, bool LANE2 = false>
+// NOISE (LANE only): the update prologue takes this filter's R from rows 4, 5 of the [6][B] buffer `noise` (fbus_set_noise)
+template <int BSF, bool TM, bool IMU32 = false, bool LANE = false, bool JOSEPH = false, bool MATLAB = false, bool LANE2 = false,
+          bool NOISE = false>
 __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh,
                                              int32_t (*sflag)[BSF], int fl, size_t b, bool live, Lane2Shared* l2 = nullptr,
-                                             const MarkerTable* tab_smem = nullptr, double* ring2 = nullptr) {
+                                             const MarkerTable* tab_smem = nullptr, double* ring2 = nullptr, const double* noise = nullptr) {
     const MarkerTable* const tab = tab_smem ? tab_smem : prm.tab;  // the second-generation lane kernel keeps a copy in shared memory
     constexpr int NT = LANE ? LANE_NT : 2 * BSF, NW = BSF / 32;
     static_assert(!LANE || BSF == 32, "the lanes-per-filter kernel has 32 filters per CTA");
     static_assert(!MATLAB || (LANE && !JOSEPH), "the MATLAB-semantics mode runs on the lanes-per-filter kernel, reference update form");
     static_assert(!LANE2 || (LANE && !MATLAB), "the second-generation lanes-per-filter kernel has the C++ semantics only");
+    static_assert(!NOISE || LANE, "the warp-specialised kernel applies R in its covariance role");
     constexpr int REC = LANE ? LX_REC : 22;  // doubles per ring slot
     constexpr int LXS = LANE2 ? L2_SHIFT : 0;  // shift of the exchange sections behind the ring
     const size_t B = prm.B;
@@ -888,8 +916,14 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
                     const MarkerConst mkc = tab->mk[req - 1];
                     if constexpr (JOSEPH) {  // 6-row factor Lc of the Joseph-form C_J and y = Lc^-1 u
                         double Cm[21], yv[6];
-                        update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, mkc, pl.y, pl.y + 3, Cm, yv,
-                                                                X + (size_t)(LXS + LX_SCR) * BSF);
+                        if constexpr (NOISE) {
+                            const MeasNoise r{noise[4 * B + b], noise[5 * B + b]};
+                            update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, r, mkc, pl.y, pl.y + 3, Cm,
+                                                                    yv, X + (size_t)(LXS + LX_SCR) * BSF);
+                        } else {
+                            update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, mkc, pl.y, pl.y + 3, Cm, yv,
+                                                                    X + (size_t)(LXS + LX_SCR) * BSF);
+                        }
 #pragma unroll
                         for (int c = 0; c < 21; ++c) X[(size_t)(LXS + LX_CM + c) * BSF] = Cm[c];
 #pragma unroll
@@ -900,7 +934,12 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
                         double L[28], Li[7], zv[7];
                         UpdHs hh;
                         update_hs<MATLAB>(n, k, mkc, pl.y, pl.y + 3, hh);
-                        update_prologue_sx<BSF, BSF, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, k, hh, L, Li, zv, X + (size_t)(LXS + LX_SCR) * BSF);
+                        if constexpr (NOISE) {
+                            const MeasNoise r{noise[4 * B + b], noise[5 * B + b]};
+                            update_prologue_sx<BSF, BSF, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, r, hh, L, Li, zv, X + (size_t)(LXS + LX_SCR) * BSF);
+                        } else {
+                            update_prologue_sx<BSF, BSF, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, k, hh, L, Li, zv, X + (size_t)(LXS + LX_SCR) * BSF);
+                        }
 #pragma unroll
                         for (int c = 0; c < 7; ++c) X[(size_t)(LXS + LX_Y + c) * BSF] = zv[c];
                     }
@@ -997,8 +1036,11 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
 // warps on schedulers 2,3 instead of 0,1) and start half a frame period late, so that one CTA's update phase (one busy
 // warp per filter group) overlaps the other's propagation phase.
 // IMU32: the IMU stream holds float32 sensor samples (FBUS_IMU_F32_SENSOR) instead of doubles
-template <int BSF, bool JOSEPH, bool IMU32 = false>  // filters per CTA; the CTA has 2*BSF threads
-__global__ void __launch_bounds__(2 * BSF) ekf_window_split_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k) {
+// NOISE: every filter has its own noise values, `noise` is the [6][B] buffer of fbus_set_noise (the other instantiations never
+// read the parameter)
+template <int BSF, bool JOSEPH, bool IMU32 = false, bool NOISE = false>  // filters per CTA; the CTA has 2*BSF threads
+__global__ void __launch_bounds__(2 * BSF) ekf_window_split_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k,
+                                                                   const double* __restrict__ noise) {
     extern __shared__ double smem[];
     __shared__ SplitShared sh;
     __shared__ int32_t sflag[3][BSF];  // [0],[1]: ring slot valid ; [2]: update requested (marker index + 1, 0 = none)
@@ -1031,8 +1073,18 @@ __global__ void __launch_bounds__(2 * BSF) ekf_window_split_kernel(const __grid_
         __shared__ uint32_t tm_slot;
         tm_base = tm_alloc_cta(&tm_slot);
     }
-    if (is_cov) cov_role<BSF, JOSEPH, TM>(prm, k, smem, sh, sflag, fl, b, live, tm_base);
-    else nominal_role<BSF, TM, IMU32>(prm, k, smem, sh, sflag, fl, b, live);
+    if constexpr (NOISE) {
+        double* sq = nullptr;
+        if constexpr (noise_q_in_smem<BSF, TM>) {
+            __shared__ double s_noise_q[4 * BSF];  // process noise of the CTA's filters: accel_n, gyro_n, accel_b, gyro_b
+            sq = s_noise_q + fl;
+        }
+        if (is_cov) cov_role<BSF, JOSEPH, TM, true>(prm, k, smem, sh, sflag, fl, b, live, tm_base, noise, sq);
+        else nominal_role<BSF, TM, IMU32>(prm, k, smem, sh, sflag, fl, b, live);
+    } else {
+        if (is_cov) cov_role<BSF, JOSEPH, TM>(prm, k, smem, sh, sflag, fl, b, live, tm_base);
+        else nominal_role<BSF, TM, IMU32>(prm, k, smem, sh, sflag, fl, b, live);
+    }
     if constexpr (TM) tm_free_cta(tm_base);
 }
 

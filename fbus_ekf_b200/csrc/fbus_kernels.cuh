@@ -5,7 +5,7 @@
 //   init_gravity_kernel K0 : FILTER::InitializeGravityAndBias (filter.cpp:256-285)
 //   refract_kernel      K3+K4: RefractionTriangulation + ComputeMarkerPose (vision.cpp:472-759)
 //   marker_pose_kernel  K4 alone
-//   stats_kernel / stats_reduce_kernel, synth_kernel, fp64_peak_kernel: measurement support.
+//   stats_kernel / stats_reduce_kernel, filter_errors_kernel, synth_kernel, fp64_peak_kernel: measurement support.
 //
 // Thread mapping: one thread per filter (or per marker); filter index fastest in every array, so a warp
 // reads/writes 32 consecutive doubles (256 B) per field.
@@ -311,6 +311,52 @@ __global__ void __launch_bounds__(128) marker_pose_kernel(const __grid_constant_
 }
 
 // ---- statistics: per-block partial sums, then a fixed-order final reduce (deterministic) ----------
+// Error of filter b against the truth, declared into the enclosing scope: ep2 = |p - p_true|^2, et2 = |dtheta|^2
+// (dtheta = 2 sign(dq_w) dq_xyz of dq = conj(q) q_true), nees = e^T P6^-1 e over (p, theta) with 6 dof, ok = false when the
+// (p, theta) block of P is not positive definite.  One definition for stats_kernel (which sums the terms) and
+// filter_errors_kernel (which writes them per filter).  A macro, not an inline function: inlining the same code changed
+// stats_kernel's register allocation and instruction schedule, and the statistics kernel is kept exactly as it was.
+#define FBUS_FILTER_ERROR_TERMS(nom, P, B, b, truth_p, truth_q)    \
+        double e[6], q[4], qt[4], dq[4]; \
+_Pragma("unroll") \
+        for (int c = 0; c < 3; ++c) e[c] = nom[(size_t)(F_P + c) * B + b] - truth_p[(size_t)c * B + b]; \
+_Pragma("unroll") \
+        for (int c = 0; c < 4; ++c) { q[c] = nom[(size_t)(F_Q + c) * B + b]; qt[c] = truth_q[(size_t)c * B + b]; } \
+        const double cq[4] = {q[0], -q[1], -q[2], -q[3]}; \
+        qmul(cq, qt, dq); \
+        const double sg = dq[0] < 0 ? -1.0 : 1.0; \
+_Pragma("unroll") \
+        for (int c = 0; c < 3; ++c) e[3 + c] = 2.0 * sg * dq[1 + c]; \
+        const int ix[6] = {0, 1, 2, 6, 7, 8}; \
+        double L[36]; \
+        bool ok = true; \
+_Pragma("unroll") \
+        for (int j = 0; j < 6; ++j) { \
+            double s = P[(size_t)pidx(ix[j], ix[j]) * B + b]; \
+_Pragma("unroll") \
+            for (int c = 0; c < j; ++c) s -= L[j * 6 + c] * L[j * 6 + c]; \
+            if (!(s > 0.0)) ok = false; \
+            const double d = sqrt(s); \
+            L[j * 6 + j] = d; \
+_Pragma("unroll") \
+            for (int i = j + 1; i < 6; ++i) { \
+                double s2 = P[(size_t)pidx(ix[i], ix[j]) * B + b]; \
+_Pragma("unroll") \
+                for (int c = 0; c < j; ++c) s2 -= L[i * 6 + c] * L[j * 6 + c]; \
+                L[i * 6 + j] = s2 / d; \
+            } \
+        } \
+        double y[6], nees = 0.0; \
+_Pragma("unroll") \
+        for (int i = 0; i < 6; ++i) { \
+            double s = e[i]; \
+_Pragma("unroll") \
+            for (int c = 0; c < i; ++c) s -= L[i * 6 + c] * y[c]; \
+            y[i] = s / L[i * 6 + i]; \
+            nees += y[i] * y[i]; \
+        } \
+        const double ep2 = e[0] * e[0] + e[1] * e[1] + e[2] * e[2]; \
+        const double et2 = e[3] * e[3] + e[4] * e[4] + e[5] * e[5];
 constexpr int STATS_BS = 128;
 __global__ void __launch_bounds__(STATS_BS) stats_kernel(const double* nom, const double* P, size_t B, const double* truth_p,
                                                          const double* truth_q, double* partial /*[grid][8]*/) {
@@ -318,46 +364,7 @@ __global__ void __launch_bounds__(STATS_BS) stats_kernel(const double* nom, cons
     const size_t b = (size_t)blockIdx.x * STATS_BS + threadIdx.x;
     double v[6] = {0, 0, 0, 0, 0, 0};  // ep2, et2, nees, n_ok, n_bad, max_ep
     if (b < B) {
-        double e[6], q[4], qt[4], dq[4];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) e[c] = nom[(size_t)(F_P + c) * B + b] - truth_p[(size_t)c * B + b];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) { q[c] = nom[(size_t)(F_Q + c) * B + b]; qt[c] = truth_q[(size_t)c * B + b]; }
-        const double cq[4] = {q[0], -q[1], -q[2], -q[3]};
-        qmul(cq, qt, dq);
-        const double sg = dq[0] < 0 ? -1.0 : 1.0;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) e[3 + c] = 2.0 * sg * dq[1 + c];
-        const int ix[6] = {0, 1, 2, 6, 7, 8};
-        double L[36];
-        bool ok = true;
-#pragma unroll
-        for (int j = 0; j < 6; ++j) {
-            double s = P[(size_t)pidx(ix[j], ix[j]) * B + b];
-#pragma unroll
-            for (int c = 0; c < j; ++c) s -= L[j * 6 + c] * L[j * 6 + c];
-            if (!(s > 0.0)) ok = false;
-            const double d = sqrt(s);
-            L[j * 6 + j] = d;
-#pragma unroll
-            for (int i = j + 1; i < 6; ++i) {
-                double s2 = P[(size_t)pidx(ix[i], ix[j]) * B + b];
-#pragma unroll
-                for (int c = 0; c < j; ++c) s2 -= L[i * 6 + c] * L[j * 6 + c];
-                L[i * 6 + j] = s2 / d;
-            }
-        }
-        double y[6], nees = 0.0;
-#pragma unroll
-        for (int i = 0; i < 6; ++i) {
-            double s = e[i];
-#pragma unroll
-            for (int c = 0; c < i; ++c) s -= L[i * 6 + c] * y[c];
-            y[i] = s / L[i * 6 + i];
-            nees += y[i] * y[i];
-        }
-        const double ep2 = e[0] * e[0] + e[1] * e[1] + e[2] * e[2];
-        const double et2 = e[3] * e[3] + e[4] * e[4] + e[5] * e[5];
+        FBUS_FILTER_ERROR_TERMS(nom, P, B, b, truth_p, truth_q)
         if (ok && isfinite(ep2) && isfinite(et2) && isfinite(nees)) {
             v[0] = ep2; v[1] = et2; v[2] = nees; v[3] = 1.0; v[5] = sqrt(ep2);
         } else {
@@ -404,6 +411,19 @@ __global__ void stats_reduce_kernel(const double* partial, int nblk, double* out
         for (int c = 0; c < 6; ++c) out[c] = red[0][c];
         out[6] = 0.0; out[7] = 0.0;
     }
+}
+
+// the per-filter terms stats_kernel sums: out[0][b] = |p - p_true|^2, [1][b] = |dtheta|^2, [2][b] = NEES (6 dof), [3][b] = 1.0
+// when all are finite and P6 is positive definite, else 0.0 (rows 0..2 then hold whatever was computed)
+__global__ void __launch_bounds__(STATS_BS) filter_errors_kernel(const double* nom, const double* P, size_t B, const double* truth_p,
+                                                                 const double* truth_q, double* out /*[4][B]*/) {
+    const size_t b = (size_t)blockIdx.x * STATS_BS + threadIdx.x;
+    if (b >= B) return;
+    FBUS_FILTER_ERROR_TERMS(nom, P, B, b, truth_p, truth_q)
+    out[b] = ep2;
+    out[B + b] = et2;
+    out[2 * B + b] = nees;
+    out[3 * B + b] = (ok && isfinite(ep2) && isfinite(et2) && isfinite(nees)) ? 1.0 : 0.0;
 }
 
 // ---- synthetic Monte-Carlo streams: Philox4x32-10 counter RNG --------------------------------------

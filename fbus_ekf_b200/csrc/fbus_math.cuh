@@ -988,6 +988,12 @@ struct CholStep<N, N> {
 struct UpdHs {
     double Hp0[9], Hp2[9], Hq[12], r[7];
 };
+// Measurement noise of one filter (rows 4, 5 of the per-filter noise buffer of fbus_set_noise).  The update functions read
+// R from `kr.Rp` / `kr.Rq` of a template type KR: DevConsts itself on the default path (the same constant loads as before),
+// this struct where every filter has its own values.
+struct MeasNoise {
+    double Rp, Rq;
+};
 template <bool MATLAB = false>
 FBUS_HD void update_hs(const Nominal& n, const DevConsts& k, const MarkerConst& mk, const double* yP, const double* yQ, UpdHs& hh) {
     double* const Hp0 = hh.Hp0;
@@ -1050,8 +1056,8 @@ FBUS_HD void update_hs(const Nominal& n, const DevConsts& k, const MarkerConst& 
         for (int i = 0; i < 4; ++i) r[3 + i] = MATLAB ? 0.0 : (yQ[i] - sg * hQ[i]);  // MeasureUpdate.m:88 zeroes the quaternion rows
     }
 }
-template <int S, int XS, class CV = Cov<S>>
-FBUS_HD void update_prologue_sx(const CV P, const DevConsts& k, const UpdHs& hh, double* L, double* Li, double* z, double* scr) {
+template <int S, int XS, class CV = Cov<S>, class KR = DevConsts>
+FBUS_HD void update_prologue_sx(const CV P, const KR& k, const UpdHs& hh, double* L, double* Li, double* z, double* scr) {
     // scr: 42 doubles of scratch with element stride XS (shared memory in the warp-specialised kernel) for X = L^-1 Hs
     const double* const Hp0 = hh.Hp0;
     const double* const Hp2 = hh.Hp2;
@@ -1156,14 +1162,15 @@ FBUS_HD void update_prologue_sx(const CV P, const DevConsts& k, const UpdHs& hh,
 // Prologue of the update: everything up to the gain factors.  Reads only the 21 entries of P6 = P[{p,theta},{p,theta}].
 // Outputs Cm = lower-packed Cholesky factor Lc of C = Hs^T S^-1 Hs and y = Lc^-1 u (u = Hs^T S^-1 r), so that
 //   (I-KH)P = P - Z^T Z with Z = Lc^T G, and dx = K r = Z^T y.
-template <int S, int XS, bool JOSEPH = false, class CV = Cov<S>>
-FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, const MarkerConst& mk, const double* yP,
+// kr: where R comes from (DevConsts or MeasNoise, see MeasNoise)
+template <int S, int XS, bool JOSEPH = false, class CV = Cov<S>, class KR = DevConsts>
+FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, const KR& kr, const MarkerConst& mk, const double* yP,
                              const double* yQ, double* Cm, double* y, double* scr) {
     double L[28], Li[7], z[7];
     {
         UpdHs hh;
         update_hs(n, k, mk, yP, yQ, hh);
-        update_prologue_sx<S, XS, CV>(P, k, hh, L, Li, z, scr);
+        update_prologue_sx<S, XS, CV>(P, kr, hh, L, Li, z, scr);
     }
 #define FBUS_L(i, j) L[(i) * ((i) + 1) / 2 + (j)]
 #define FBUS_X(i) scr[(i) * XS]
@@ -1224,7 +1231,7 @@ FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, c
                 FBUS_UNROLL
                 for (int c = 0; c < 6; ++c) s -= CP[i * 6 + c] * ((c >= j) ? FBUS_C(c, j) : FBUS_C(j, c));
                 FBUS_UNROLL
-                for (int c = 0; c < 7; ++c) s -= ((c < 3) ? k.Rp : k.Rq) * Y[c * 6 + i] * Y[c * 6 + j];
+                for (int c = 0; c < 7; ++c) s -= ((c < 3) ? kr.Rp : kr.Rq) * Y[c * 6 + i] * Y[c * 6 + j];
                 CJ[i * (i + 1) / 2 + j] = s;
             }
         FBUS_UNROLL
@@ -1246,6 +1253,12 @@ FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, c
         }
     }
 #undef FBUS_C
+}
+// R from the constants
+template <int S, int XS, bool JOSEPH = false, class CV = Cov<S>>
+FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, const MarkerConst& mk, const double* yP,
+                             const double* yQ, double* Cm, double* y, double* scr) {
+    update_prologue<S, XS, JOSEPH, CV>(P, n, k, k, mk, yP, yQ, Cm, y, scr);
 }
 
 // rows 0..2 of Z = Lc^T G from the current P (G = rows {0,1,2,6,7,8} of P)
@@ -1641,15 +1654,15 @@ FBUS_HD void update_onepass_blk(const CV P, Nominal& n, const double* Cm, const 
     }
 }
 
-// stash: 54 doubles of scratch with stride XS (nullptr: a private array)
-template <int S, int JMODE = -1, int XS = 1, class CV = Cov<S>>
-FBUS_HD void measurement_update(const CV P, Nominal& n, const DevConsts& k, const MarkerConst& mk, const double* yP,
-                                const double* yQ, double* stash = nullptr, bool on = true) {
+// stash: 54 doubles of scratch with stride XS (nullptr: a private array); kr: where R comes from (DevConsts or MeasNoise)
+template <int S, int JMODE = -1, int XS = 1, class CV = Cov<S>, class KR = DevConsts>
+FBUS_HD void measurement_update(const CV P, Nominal& n, const DevConsts& k, const KR& kr, const MarkerConst& mk, const double* yP,
+                                const double* yQ, double* stash, bool on) {
     double Cm[21], y[6];
     {
         double xloc[42];  // X = L^-1 Hs stays private
-        if (JMODE == 1 || (JMODE < 0 && (k.flags & 1))) update_prologue<S, 1, true>(P, n, k, mk, yP, yQ, Cm, y, xloc);
-        else update_prologue<S, 1, false>(P, n, k, mk, yP, yQ, Cm, y, xloc);
+        if (JMODE == 1 || (JMODE < 0 && (k.flags & 1))) update_prologue<S, 1, true>(P, n, k, kr, mk, yP, yQ, Cm, y, xloc);
+        else update_prologue<S, 1, false>(P, n, k, kr, mk, yP, yQ, Cm, y, xloc);
     }
     if (!on) {  // lane without an update inside a warp that must stay convergent: zero gain, P and the state keep their values
         FBUS_UNROLL
@@ -1779,6 +1792,12 @@ FBUS_HD void measurement_update(const CV P, Nominal& n, const DevConsts& k, cons
         FBUS_UNROLL
         for (int i = 0; i < 4; ++i) n.q[i] = qn[i];
     }
+}
+// R from the constants
+template <int S, int JMODE = -1, int XS = 1, class CV = Cov<S>>
+FBUS_HD void measurement_update(const CV P, Nominal& n, const DevConsts& k, const MarkerConst& mk, const double* yP,
+                                const double* yQ, double* stash = nullptr, bool on = true) {
+    measurement_update<S, JMODE, XS, CV>(P, n, k, k, mk, yP, yQ, stash, on);
 }
 
 }  // namespace fbus

@@ -194,6 +194,38 @@ class BatchFilter:
         self._ck(self._lib.fbus_stats(self._h, tp, tq, mem, capi.dptr(out) if want_host else None, out_dev_ptr))
         return out
 
+    def SetNoise(self, noise=None, mem: int = capi.FBUS_MEM_HOST):
+        """Per-filter noise covariances (fbus_set_noise): float64 [6][B] numpy array, rows in capi.NOISE_FIELDS order, or a
+        device pointer (mem = FBUS_MEM_DEVICE) to such an array.  None returns the handle to the config's values."""
+        if noise is None:
+            self._ck(self._lib.fbus_set_noise(self._h, None, mem))
+            return
+        if mem == capi.FBUS_MEM_HOST:
+            assert isinstance(noise, np.ndarray) and noise.dtype == np.float64 and noise.flags["C_CONTIGUOUS"], "float64 C-contiguous array"
+            assert noise.shape == (capi.FBUS_NOISE_FIELDS, self.batch), noise.shape
+            self._ck(self._lib.fbus_set_noise(self._h, noise.ctypes.data, mem))
+        else:
+            self._ck(self._lib.fbus_set_noise(self._h, int(noise), mem))
+
+    def FilterErrors(self, truth_p, truth_q, mem: int = capi.FBUS_MEM_HOST, out=None, out_mem: int = capi.FBUS_MEM_HOST):
+        """Per-filter error terms (fbus_filter_errors) -> [4][B]: |p - p_true|^2, |dtheta|^2, NEES (6 dof), finite flag.
+        truth_p [3][B], truth_q [4][B] float64 numpy arrays (or device pointers with mem = FBUS_MEM_DEVICE).  Output: a new
+        numpy array, the given numpy array, or the given device pointer (out_mem = FBUS_MEM_DEVICE)."""
+        if mem == capi.FBUS_MEM_HOST:
+            for a, n in ((truth_p, 3), (truth_q, 4)):
+                assert isinstance(a, np.ndarray) and a.dtype == np.float64 and a.flags["C_CONTIGUOUS"] and a.shape == (n, self.batch)
+            tp, tq = truth_p.ctypes.data, truth_q.ctypes.data
+        else:
+            tp, tq = int(truth_p), int(truth_q)
+        if out_mem == capi.FBUS_MEM_HOST:
+            if out is None:
+                out = np.empty((4, self.batch))
+            assert out.dtype == np.float64 and out.flags["C_CONTIGUOUS"] and out.shape == (4, self.batch)
+            self._ck(self._lib.fbus_filter_errors(self._h, tp, tq, mem, out.ctypes.data, out_mem))
+        else:
+            self._ck(self._lib.fbus_filter_errors(self._h, tp, tq, mem, int(out), out_mem))
+        return out
+
     def SynthStreams(self, spec: capi.SynthSpec, imu_ptr: int, det_id_ptr: int, det_pose_ptr: int, bias_ptr: int | None = None):
         self._ck(self._lib.fbus_synth_streams(self._h, C.byref(spec), imu_ptr, det_id_ptr, det_pose_ptr, bias_ptr))
 

@@ -34,7 +34,8 @@
 extern "C" {
 #endif
 
-#define FBUS_ABI_VERSION 3 /* 2: fbus_config.imu_g / gn_tol, fbus_imu_stream.format, fbus_iir_prefilter; 3: fbus_stats_allreduce*, FBUS_E_NCCL */
+#define FBUS_ABI_VERSION 3 /* 2: fbus_config.imu_g / gn_tol, fbus_imu_stream.format, fbus_iir_prefilter; 3: fbus_stats_allreduce*, FBUS_E_NCCL;
+                              added within 3 (no struct changed): fbus_set_noise, fbus_filter_errors */
 
 /* error codes */
 #define FBUS_OK 0
@@ -311,6 +312,18 @@ int fbus_marker_pose(fbus_handle* h, const double* corners3d, size_t n, double* 
    stretch). */
 int fbus_iir_prefilter(fbus_handle* h, const fbus_imu_stream* in, size_t first, size_t count, double* out, int32_t out_mem);
 
+/* ---- per-filter noise values ------------------------------------------------------------- */
+
+/* rows of a per-filter noise array, in fbus_config order */
+#define FBUS_NOISE_FIELDS 6 /* accel_n_cov, gyro_n_cov, accel_b_cov, gyro_b_cov, pos_n_cov, quat_n_cov */
+/* Gives every filter its own noise covariances: noise is [FBUS_NOISE_FIELDS][B] doubles (mem as given), row f holding the
+   fbus_config field f of each filter.  The array is copied into a handle-owned device buffer (allocated on the first call,
+   freed by fbus_destroy), and from the next stepping call on (fbus_step_windows, fbus_propagate, fbus_update,
+   fbus_reset_state, the init calls) filter b uses column b in place of the config's six values, used as given like
+   fbus_config's.  noise = NULL returns the handle to the config's values.  State, status and the continuation rule of
+   fbus_step_windows are untouched: a call between two continued calls takes effect from the next call on. */
+int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem);
+
 /* ---- state access ------------------------------------------------------------------------- */
 
 int fbus_get_state(fbus_handle* h, fbus_state_soa* out); /* synchronises */
@@ -327,6 +340,13 @@ int fbus_clear_status(fbus_handle* h);
    without a host round trip; out_host (optional) is HOST. */
 int fbus_stats(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem,
                double* out_host, double* out_dev);
+/* Per-filter error terms, the ones fbus_stats sums: out is [4][B] (out_mem as given) with
+   out[0][b] = |p - p_true|^2, out[1][b] = |dtheta|^2, out[2][b] = NEES over (p,theta) (6 dof), out[3][b] = 1.0 when the three
+   are finite and the (p,theta) block of P is positive definite, else 0.0 (rows 0..2 then hold whatever was computed).
+   fbus_stats entries 0..4 are the sums of rows 0..2 over filters with flag 1 and the counts of flags 1 and 0 (up to
+   summation order); entry 5 is exactly the maximum of sqrt(row 0) over filters with flag 1.  truth_p [3][B], truth_q [4][B]
+   (mem as given).  Synchronises when out is HOST. */
+int fbus_filter_errors(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem, double* out, int32_t out_mem);
 /* Combine rule of the per-shard vectors (SURVEY 8e: what the multi-GPU driver applies with its all-reduce; here for callers
    that gather the vectors themselves -- several handles in one process, MPI): parts is [n_parts][FBUS_NSTATS] on the HOST;
    out[0..4] = sums over the parts, out[5] = maximum, out[6..7] = 0.  Pure host code, needs no handle. */
