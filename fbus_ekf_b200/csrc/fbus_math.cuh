@@ -948,8 +948,12 @@ FBUS_HD void vision_pose(const DevConsts& k, const MarkerConst& mk, const double
 //   (I-KH)P = P - G^T C G,  C = Hs^T S^-1 Hs = Lc Lc^T  ->  P' = P - Z^T Z,  Z = Lc^T G.
 // Z is applied in two half-rank sweeps (rows 0..2 then 3..5) so that only 54 doubles are live;
 // G's theta rows are rebuilt between the sweeps (see DESIGN.md "update without scratch").
-// S is SPD with cond <= ~13 on the reference's logs, so Cholesky replaces the reference's LDLT
-// (filter.cpp:711) to ~1e-15.
+// S is SPD, so Cholesky replaces the reference's LDLT (filter.cpp:711).  Measured against a 50-digit evaluation of one update
+// (tests/test_precision_host.py, host build of this header), the error of the updated (p, theta) block whitened by its exact
+// value stays within 1.2 to 3.4x of the dense double oracle's own error for R from 1e-3 down to 1e-12: 3e-16 at the default
+// R = 1e-3, 3e-12 at the noise sweep's corner (pos 1e-8, quat 1e-7), 8e-10 at 1e-10 and 7e-8 at 1e-12.  Both forms lose about
+// eps * |P6 before| / |P6 after| to the cancellation in P - K H P; tests/test_gpu_precision.py holds every kernel form to 8x the
+// oracle's error and to 1e-9 on the sweep's range (R >= 1e-8).
 // ------------------------------------------------------------------------------------------------
 // In-place Cholesky of a packed lower-triangular matrix (row-major packed: L[i*(i+1)/2 + j]); also returns the
 // reciprocal diagonal.  Template recursion instead of a loop over columns: nvcc does not fully unroll the
@@ -1197,6 +1201,9 @@ FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, c
         // FBUS_FLAG_JOSEPH (compile-time variant so that the default path carries none of this code): Joseph-form covariance update  P' = (I-KH) P (I-KH)^T + K R K^T  evaluated in the same reduced
         // space.  With K = G^T Hs^T S^-1 it equals  P - G^T C_J G,  C_J = 2C - C P6 C - D,  D = Y^T R Y,  Y = S^-1 Hs
         // (C P6 C + D = C in exact arithmetic, so C_J = C up to rounding; the default is the reference's (I-KH)P).
+        // P - G^T C_J G subtracts from P like the standard form, so this has the standard form's accuracy, not the dense Joseph
+        // form's: at the sweep's corner (R = 1e-8 / 1e-7) the whitened P6 error is 6e-12 against 2e-15 for the oracle's dense
+        // (I-KH) P (I-KH)^T + K R K^T, and 7e-8 against 7e-16 at R = 1e-12 (host build, tests/test_precision_host.py).
         double Y[42];  // S^-1 Hs = L^-T X  (back substitution)
         FBUS_UNROLL
         for (int i = 6; i >= 0; --i)

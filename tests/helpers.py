@@ -45,6 +45,34 @@ def cov_close(P, Pref, rtol=1e-9):
     return bool(ok_abs and ok_rel), worst
 
 
+IX6 = [0, 1, 2, 6, 7, 8]  # (position, attitude): the block of P that the 6-dof NEES inverts
+
+
+def _cov18(P):
+    """one filter's covariance ([324] or 18x18, float64 or an object array of mpmath numbers) -> 18x18 object array of mpf"""
+    import mp_reference as mpr
+    return mpr.mpa(np.asarray(P).reshape(18, 18))
+
+
+def cov_whitened_err(P, Pref):
+    """max |L^-1 (P6 - P6ref) L^-T| with L = chol(P6ref), P6 = P[IX6, IX6], evaluated in mpmath.  It bounds the relative
+    error of any e^T P6^-1 e (NEES) computed from P6 instead of P6ref, whatever P6's scale and conditioning, which cov_close's
+    max|P|-scaled measure does not.  P, Pref: one filter, [324] or 18x18; Pref may be an mpmath object array (exact)."""
+    import mp_reference as mpr
+    D = (_cov18(P) - _cov18(Pref))[np.ix_(IX6, IX6)]
+    Li = mpr._inv(mpr._chol(_cov18(Pref)[np.ix_(IX6, IX6)]))
+    return float(np.abs(mpr.to_np(Li @ D @ Li.T)).max())
+
+
+def cov_corr_err(P, Pref):
+    """max |P_ij - Pref_ij| / sqrt(Pref_ii Pref_jj) over all 18x18 entries: the error relative to the correlation scale of each
+    entry, so small variances (a converged pose block) weigh as much as the gravity block.  Same arguments as cov_whitened_err."""
+    import mp_reference as mpr
+    A, B = _cov18(P), _cov18(Pref)
+    d = np.sqrt(np.abs(np.diag(mpr.to_np(B))))
+    return float((np.abs(mpr.to_np(A - B)) / np.outer(d, d)).max())
+
+
 def state_close(a, b, rtol=1e-9, fields=NOM):
     worst = 0.0
     ok = True

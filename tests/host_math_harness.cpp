@@ -50,6 +50,21 @@ int hm_update(const fbus_config* cfg, double* P171, double* nom, int marker_id, 
     nom_to(n, nom);
     return 0;
 }
+
+// the Joseph-form instantiation (FBUS_FLAG_JOSEPH) whatever cfg->flags says
+int hm_update_joseph(const fbus_config* cfg, double* P171, double* nom, int marker_id, const double* yP, const double* yQ) {
+    DevConsts k;
+    MarkerTable tab;
+    if (make_dev_consts(cfg, &k, &tab)) return -1;
+    const int m = find_marker(k, &tab, marker_id);
+    if (m < 0) return -2;
+    Nominal n;
+    nom_from(nom, n);
+    Cov<1> P{P171};
+    measurement_update<1, 1>(P, n, k, tab.mk[m], yP, yQ);
+    nom_to(n, nom);
+    return 0;
+}
 }
 
 extern "C" int hm_update_coop(const fbus_config* cfg, double* P171, double* nom, int marker_id, const double* yP, const double* yQ) {

@@ -3,7 +3,7 @@ them, on every form of the window kernel.  Streams come from fbus_synth_streams;
 import numpy as np
 import pytest
 
-from helpers import cov_close, random_states, state_close
+from helpers import cov_close, cov_whitened_err, random_states, state_close
 
 pytestmark = pytest.mark.gpu
 
@@ -106,6 +106,10 @@ def _oracle_close(run, ref):
     assert ok, w
     ok, w = cov_close(st["P"], so["P"], RTOL)
     assert ok, w
+    # cov_close scales by max|P| (the gravity block); the NEES block is checked on its own scale
+    for b in range(st["P"].shape[1]):
+        w = cov_whitened_err(st["P"][:, b], so["P"][:, b])
+        assert w <= RTOL, (b, w)
     assert np.abs(tr - tro).max() <= RTOL
 
 
