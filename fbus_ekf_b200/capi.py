@@ -25,6 +25,7 @@ FBUS_ST_INIT_FAILED, FBUS_ST_RESET_SKIPPED, FBUS_ST_RESET_DONE, FBUS_ST_UPDATE_S
 FBUS_ST_NONFINITE, FBUS_ST_NO_DETECTION, FBUS_ST_MARKER_REJECTED = 0x10, 0x20, 0x40
 FBUS_FLAG_JOSEPH = 0x1
 FBUS_FLAG_MATLAB = 0x2
+FBUS_FLAG_ALL_MARKERS = 0x4  # every known marker of a frame updates the filter in turn (include/fbus_ekf.h)
 FBUS_MAX_MARKERS = 16
 FBUS_NSTATS = 8
 # rows of a per-filter noise array (fbus_set_noise), in fbus_config order

@@ -175,7 +175,14 @@ int launch_window_t(fbus_handle* h, WinParams& prm) {
     const unsigned grid = (unsigned)((h->B + WIN_BS - 1) / WIN_BS);
     const bool jo = (h->k.flags & FBUS_FLAG_JOSEPH) != 0, f32 = prm.imu32 != nullptr;
     const double* const nz = NOISE ? (const double*)h->noise.p : nullptr;
-    if (h->k.flags & FBUS_FLAG_MATLAB) {  // MATLAB-semantics mode: the lanes-per-filter kernel at any batch size
+    if (h->k.flags & FBUS_FLAG_ALL_MARKERS) {  // every marker of a frame: the first-generation lanes-per-filter kernel at any batch size
+        const unsigned g32 = (unsigned)((h->B + 31) / 32);
+        if (f32) {
+            if (jo) ekf_window_lane_kernel<true, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+            else ekf_window_lane_kernel<false, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        else ekf_window_lane_kernel<false, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+    } else if (h->k.flags & FBUS_FLAG_MATLAB) {  // MATLAB-semantics mode: the lanes-per-filter kernel at any batch size
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
         if (f32) ekf_window_lane_kernel<false, true, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
         else ekf_window_lane_kernel<false, false, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
@@ -236,6 +243,10 @@ cudaError_t set_window_smem_limits() {
     set((const void*)ekf_window_lane_kernel<true, true, false, NOISE>, LANE_SMEM);
     set((const void*)ekf_window_lane_kernel<false, false, true, NOISE>, LANE_SMEM);
     set((const void*)ekf_window_lane_kernel<false, true, true, NOISE>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<false, false, false, NOISE, true>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<true, false, false, NOISE, true>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<false, true, false, NOISE, true>, LANE_SMEM);
+    set((const void*)ekf_window_lane_kernel<true, true, false, NOISE, true>, LANE_SMEM);
     set((const void*)ekf_window_lane2_kernel<false, false, NOISE>, LANE2_SMEM);
     set((const void*)ekf_window_lane2_kernel<true, false, NOISE>, LANE2_SMEM);
     set((const void*)ekf_window_lane2_kernel<false, true, NOISE>, LANE2_SMEM);
@@ -247,6 +258,7 @@ int stage_det(fbus_handle* h, const fbus_det_frames* det, size_t w0, size_t w1, 
     if (!det || det->batch != h->B || w1 > det->n_frames || w0 > w1 || det->max_markers == 0 || !det->t || !det->id || !det->pose)
         return fail(h, FBUS_E_BADARG, "bad detection frames");
     const size_t m = det->max_markers, B = h->B, nw = w1 - w0;
+    if ((h->k.flags & FBUS_FLAG_ALL_MARKERS) && m > 32) return fail(h, FBUS_E_BADARG, "FBUS_FLAG_ALL_MARKERS: max_markers > 32");
     // timestamps are always host memory; stage only the frames of this call, re-based to index 0
     const double* dt;
     int rc = stage(h, h->det_t, det->t + w0, nw, FBUS_MEM_HOST, &dt);
@@ -317,6 +329,10 @@ int fbus_create(fbus_handle** out, const fbus_config* cfg, int device, size_t ba
     if ((cfg->flags & FBUS_FLAG_MATLAB) && (cfg->flags & FBUS_FLAG_JOSEPH)) {
         delete h;
         return fail(nullptr, FBUS_E_BADARG, "fbus_create: FBUS_FLAG_MATLAB and FBUS_FLAG_JOSEPH cannot be combined");
+    }
+    if ((cfg->flags & FBUS_FLAG_MATLAB) && (cfg->flags & FBUS_FLAG_ALL_MARKERS)) {
+        delete h;
+        return fail(nullptr, FBUS_E_BADARG, "fbus_create: FBUS_FLAG_MATLAB and FBUS_FLAG_ALL_MARKERS cannot be combined");
     }
     if (make_dev_consts(cfg, &h->k, &h->tab) != FBUS_OK) {
         delete h;
@@ -540,6 +556,8 @@ static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const 
                               size_t w0, size_t w1, double* trace, int32_t trace_mem, bool resume, size_t chunk_frames) {
     const size_t B = h->B, nw = w1 - w0, m = det->max_markers;
     if (det->batch != B || w1 > det->n_frames || m == 0 || !det->t || !det->id || !det->pose) return fail(h, FBUS_E_BADARG, "bad detection frames");
+    // the kernel keeps a frame's update slots as a 32-bit mask
+    if ((h->k.flags & FBUS_FLAG_ALL_MARKERS) && m > 32) return fail(h, FBUS_E_BADARG, "FBUS_FLAG_ALL_MARKERS: max_markers > 32");
     const size_t s0 = win_off[w0], s1 = win_off[w1];
     const bool imu_host = imu->mem == FBUS_MEM_HOST, det_host = det->mem == FBUS_MEM_HOST;
     WinParams prm;

@@ -138,7 +138,9 @@ __device__ __forceinline__ void lane_apply_Fu1(double* x, const double* A, const
 
 // COVARIANCE lanes: warp cw (0..10) holds filters 3cw .. 3cw+2 of the CTA, lane = 9*g + l
 // NOISE: q0, q1 come from this filter's row of the [6][B] buffer `noise` (fbus_set_noise) instead of k.Qd
-template <bool JOSEPH, bool NOISE = false>
+// ALL: FBUS_FLAG_ALL_MARKERS -- after the first update of a frame, further update rounds follow until no filter of the CTA
+// requests one (nominal_role posts one marker per filter and round)
+template <bool JOSEPH, bool NOISE = false, bool ALL = false>
 __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh, int32_t (*sflag)[32],
                                               int cw, int lane, const double* noise = nullptr) {
     constexpr int NT = LANE_NT;
@@ -219,6 +221,8 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
         }
         cta_bar<NT>();  // (r) update requests posted
         if (sh.any_upd[0]) {
+            // ALL: one round per posted request (nominal_role), until a round without any
+            do {
             const bool req = act && sflag[2][f] != 0;
             // the 6x6 block of the p / theta rows and columns for the prologue: lanes l in {0,1,2,6,7,8} own its columns
             if (req && (l < 3 || l >= 6)) {
@@ -293,6 +297,7 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
             }
             __syncwarp();
             cta_bar<NT>();  // (d) dx posted
+            } while (ALL && (cta_bar<NT>(), sh.any_upd[0] != 0));  // (r) of the next round: does any filter request one?
         }
     }
     if (live) {  // upper triangle back: column j is stored by its owner for rows i <= j
@@ -306,7 +311,8 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
 
 // NOISE: every filter has its own noise values, `noise` is the [6][B] buffer of fbus_set_noise (the other instantiations never
 // read the parameter)
-template <bool JOSEPH, bool IMU32, bool MATLAB = false, bool NOISE = false>
+// ALL: FBUS_FLAG_ALL_MARKERS, every known marker of a frame updates the filter in turn (include/fbus_ekf.h)
+template <bool JOSEPH, bool IMU32, bool MATLAB = false, bool NOISE = false, bool ALL = false>
 __global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k,
                                                                      const double* __restrict__ noise) {
     extern __shared__ double smem[];
@@ -314,15 +320,15 @@ __global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __gri
     __shared__ int32_t sflag[3][32];
     const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (wi < 11) {
-        if constexpr (NOISE) lane_cov_role<JOSEPH, true>(prm, k, smem, sh, sflag, wi, lane, noise);
-        else lane_cov_role<JOSEPH>(prm, k, smem, sh, sflag, wi, lane);
+        if constexpr (NOISE) lane_cov_role<JOSEPH, true, ALL>(prm, k, smem, sh, sflag, wi, lane, noise);
+        else lane_cov_role<JOSEPH, false, ALL>(prm, k, smem, sh, sflag, wi, lane);
     } else {
         const size_t b0 = (size_t)blockIdx.x * 32 + lane;
         const bool live = b0 < prm.B;
         if constexpr (NOISE)
-            nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live, nullptr,
-                                                                              nullptr, nullptr, noise);
-        else nominal_role<32, false, IMU32, true, JOSEPH, MATLAB>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live);
+            nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, true, ALL>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live,
+                                                                                   nullptr, nullptr, nullptr, noise);
+        else nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, false, ALL>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live);
     }
 }
 

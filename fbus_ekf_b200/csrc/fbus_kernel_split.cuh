@@ -291,9 +291,13 @@ struct FramePlan {
     double t_init;           // time of the last IMU sample not later than the initialising frame (preImuTime, FBUS_EKF.m:175)
     double t_img_new;        // preImgTime after this frame
     bool set_t_img;
+    // FBUS_FLAG_ALL_MARKERS only (dead in the other instantiations): slots of the frame's further updates, bit s = slot s; their
+    // poses are read again from the detection buffers when their round comes
+    uint32_t extra;
 };
 
-template <int BSF>
+// ALL: FBUS_FLAG_ALL_MARKERS -- pl.extra lists the frame's other known markers (max_markers <= 32, checked by the host)
+template <int BSF, bool ALL = false>
 __device__ __forceinline__ void plan_frame(const WinParams& prm, const DevConsts& k, const MarkerTable* tab, uint32_t w, size_t b, bool live,
                                            uint32_t cursor, double n_t, int inited, int& prev_id, int& status, FramePlan& pl) {
     const size_t B = prm.B;
@@ -417,6 +421,26 @@ __device__ __forceinline__ void plan_frame(const WinParams& prm, const DevConsts
             for (int c = 0; c < 7; ++c) pl.y[c] = pp[(size_t)c * B];
         } else {
             status |= FBUS_ST_UPDATE_SKIPPED;
+        }
+    }
+    if constexpr (ALL) {  // every other slot with a known id, in slot order
+        pl.extra = 0u;
+        if (do_update && n_det > 0) {
+            for (int s = 0; s < prm.m; ++s) {
+                if (s == idx_upd) continue;
+                const int id = prm.det_id[((size_t)w * prm.m + s) * B + b];
+                if (id < 0) continue;
+                if (find_marker(k, tab, id) >= 0) pl.extra |= 1u << s;
+                else status |= FBUS_ST_UPDATE_SKIPPED;
+            }
+        }
+        if (pl.req == 0 && pl.extra != 0u) {  // the chosen marker is unknown: the first other one takes its round (prev_id unchanged)
+            const size_t slot = (size_t)w * prm.m + (__ffs(pl.extra) - 1);
+            pl.extra &= pl.extra - 1u;
+            pl.req = find_marker(k, tab, prm.det_id[slot * B + b]) + 1;
+            const double* pp = prm.det_pose + slot * 7 * B + b;
+#pragma unroll
+            for (int c = 0; c < 7; ++c) pl.y[c] = pp[(size_t)c * B];
         }
     }
 }
@@ -592,8 +616,11 @@ struct P6View {
 // state-only prologue (predicted measurement, Hs, S, the gain factors) from the published P6 and the error-state
 // injection, the covariance lanes run the sweep P -= Z^T Z and dx = Z^T y.
 // NOISE (LANE only): the update prologue takes this filter's R from rows 4, 5 of the [6][B] buffer `noise` (fbus_set_noise)
+// ALL (first-generation LANE only): FBUS_FLAG_ALL_MARKERS -- the update hand-off (r) (p) (c) (d) repeats, one marker per filter and
+// round (the planned one, then pl.extra in slot order), each at the state the previous injection left, until a round in which no
+// filter of the CTA posts a request; the next frame's plan is made in the first round only
 template <int BSF, bool TM, bool IMU32 = false, bool LANE = false, bool JOSEPH = false, bool MATLAB = false, bool LANE2 = false,
-          bool NOISE = false>
+          bool NOISE = false, bool ALL = false>
 __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh,
                                              int32_t (*sflag)[BSF], int fl, size_t b, bool live, Lane2Shared* l2 = nullptr,
                                              const MarkerTable* tab_smem = nullptr, double* ring2 = nullptr, const double* noise = nullptr) {
@@ -603,6 +630,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
     static_assert(!MATLAB || (LANE && !JOSEPH), "the MATLAB-semantics mode runs on the lanes-per-filter kernel, reference update form");
     static_assert(!LANE2 || (LANE && !MATLAB), "the second-generation lanes-per-filter kernel has the C++ semantics only");
     static_assert(!NOISE || LANE, "the warp-specialised kernel applies R in its covariance role");
+    static_assert(!ALL || (LANE && !LANE2 && !MATLAB), "the all-markers mode runs on the first-generation lanes-per-filter kernel, C++ semantics");
     constexpr int REC = LANE ? LX_REC : 22;  // doubles per ring slot
     constexpr int LXS = LANE2 ? L2_SHIFT : 0;  // shift of the exchange sections behind the ring
     const size_t B = prm.B;
@@ -638,7 +666,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
     double t_img = MATLAB ? prm.nom[(size_t)F_TIMG * B + b] : 0.0;  // preImgTime (FBUS_EKF.m:144)
     auto plan = [&](uint32_t wf, FramePlan& out) {
         if constexpr (MATLAB) plan_frame_matlab<BSF>(prm, k, tab, wf, b, live, cursor, t_img, inited, prev_id, status, out);
-        else plan_frame<BSF>(prm, k, tab, wf, b, live, cursor, n.t, inited, prev_id, status, out);
+        else plan_frame<BSF, ALL>(prm, k, tab, wf, b, live, cursor, n.t, inited, prev_id, status, out);
         if constexpr (LANE2) {
             // lanes past the batch mirror the last filter for their reads; in this kernel they neither propagate nor update, so
             // that a small batch (the live single-filter case) leaves the covariance warps of the unused slots asleep
@@ -691,7 +719,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
         const bool do_prop = pl.do_prop;
         const uint32_t p_first = pl.p_first, p_end = pl.p_end;
         const double t_end = pl.t_end;
-        const int req = pl.req;
+        int req = pl.req;  // marker index + 1 of this round's update (ALL: changes from round to round)
 
         // ---- F3 BatchImuProcessing (filter.cpp:483-531): one sample ahead of the covariance warp -------------
         const int fp = (int)((w - prm.w0) & 1u);  // copy of the range table this frame uses (see SplitShared)
@@ -887,6 +915,10 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
             if (fused && do_prop) cursor = consumed;
         }
 
+        FramePlan nx;
+        nx.do_prop = nx.apply_init = nx.apply_reset = false;
+        nx.req = 0;
+        for (uint32_t round = 0;; ++round) {
         // ---- F4 ObservationUpdate (filter.cpp:622-739): post the request (into the ring slot the covariance warp is
         //      not reading), the covariance warp does the algebra ------------------------------------------------
         if (req && !LANE) {
@@ -949,10 +981,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
             }
         }
         // ---- while the update runs: the next window's first IMU sample and the next frame's plan ---------------
-        FramePlan nx;
-        nx.do_prop = nx.apply_init = nx.apply_reset = false;
-        nx.req = 0;
-        if (w + 1 < prm.w1) {
+        if (w + 1 < prm.w1 && (!ALL || round == 0)) {
             if (!LANE2 && fused && cursor < prm.win_off[prm.w1]) {  // (the second-generation lane kernel loads the samples in its covariance warps)
                 pf_i = cursor;
                 pf_st = prm.imu_t[cursor];
@@ -984,6 +1013,21 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
                     for (int c = 0; c < 4; ++c) n.q[c] = X[(size_t)(26 + c) * BSF];  // rotmatI2G deliberately NOT refreshed (A.3-2)
                 }
             }
+        }
+        if constexpr (!ALL) {
+            break;
+        } else {  // FBUS_FLAG_ALL_MARKERS: this filter's next marker of the frame, if any; a round nobody requested ends the frame
+            if (!any) break;
+            req = 0;
+            if (pl.extra) {
+                const size_t slot = (size_t)w * prm.m + (__ffs(pl.extra) - 1);
+                pl.extra &= pl.extra - 1u;
+                req = find_marker(k, tab, prm.det_id[slot * B + b]) + 1;
+                const double* pp = prm.det_pose + slot * 7 * B + b;
+#pragma unroll
+                for (int c = 0; c < 7; ++c) pl.y[c] = pp[(size_t)c * B];
+            }
+        }
         }
         // ---- trace row: the data/fusion.txt record (filter.cpp:241-246) -------------------------
         if (prm.trace && live) {

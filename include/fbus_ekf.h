@@ -92,6 +92,25 @@ extern "C" {
                                 lanes-per-filter window kernel at any batch size; not combinable with FBUS_FLAG_JOSEPH.
                                 Checked against oracle/fbus_oracle_matlab.py (a NumPy restatement of the .m files; "parity
                                 unpinned": no MATLAB here). */
+#define FBUS_FLAG_ALL_MARKERS 0x4 /* opt-in: every detected marker of a frame updates the filter, not only the nearest one.
+    1. Every frame that gets a measurement update in the reference's path (the fused path of fbus_step_windows after reset
+       and propagation; fbus_update) gets a SEQUENCE of 7-row updates.  The first uses exactly the marker the reference
+       chooses (nearest, with the marker_switch_thres hysteresis against prev_marker_id; prev_marker_id is updated as
+       always); if that marker is known, this step is bit-for-bit the default update.
+    2. Every other slot of the frame follows in slot order if its id is >= 0 and in the marker map: a separate 7-row update
+       with the reference's measurement model and quaternion sign choice, linearised at the state the previous update left
+       (sequential updates with injection in between).  Covariance form (I-KH)P, or the reduced Joseph form under
+       FBUS_FLAG_JOSEPH; R is the config's or, under fbus_set_noise, the filter's own.
+    3. A slot whose id is unknown is skipped and sets FBUS_ST_UPDATE_SKIPPED.  If the chosen marker is unknown, the other
+       known markers are still applied and prev_marker_id stays unchanged, as in the reference.
+    4. Init, reset and the vision-only pose still use the nearest marker only; trace rows, status bits and the continuation
+       rule of fbus_step_windows are unchanged.
+    5. With at most one known detection per frame the results equal the default mode's.
+    6. Not combinable with FBUS_FLAG_MATLAB (fbus_create returns FBUS_E_BADARG); combines with FBUS_FLAG_JOSEPH,
+       fbus_set_noise and both IMU element formats.
+    7. The kernel keeps a frame's update slots as a 32-bit mask: with this flag the stepping calls reject
+       max_markers > 32 with FBUS_E_BADARG (the default mode takes any max_markers).
+    Runs on the first-generation lanes-per-filter window kernel at any batch size. */
 
 /*
  * Per-run constants.  Mirrors EkfParam / RefractInfo / CameraInfo.T_SC / MarkerPoseServer
