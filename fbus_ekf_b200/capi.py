@@ -100,6 +100,13 @@ class SynthSpec(C.Structure):
                 ("sigma_pos", C.c_double), ("sigma_quat", C.c_double), ("seed", C.c_uint64), ("filter_offset", C.c_uint64)]
 
 
+class CornerSpec(C.Structure):
+    """fbus_corner_spec (fbus_synth_corners)"""
+    _fields_ = [("n_frames", C.c_size_t), ("max_markers", C.c_size_t), ("base_pose", c_double_p), ("base_id", c_int32_p),
+                ("underwater", C.c_int32), ("reserved", C.c_int32), ("sigma_corner", C.c_double), ("p_drop", C.c_double),
+                ("p_outlier", C.c_double), ("sigma_outlier", C.c_double), ("seed", C.c_uint64), ("filter_offset", C.c_uint64)]
+
+
 STATE_FIELDS = (("t", 1, np.float64), ("q", 4, np.float64), ("R", 9, np.float64), ("p", 3, np.float64),
                 ("v", 3, np.float64), ("ba", 3, np.float64), ("bg", 3, np.float64), ("g", 3, np.float64),
                 ("pv", 3, np.float64), ("qv", 4, np.float64), ("P", 324, np.float64),
@@ -176,6 +183,8 @@ def lib() -> C.CDLL:
         "fbus_stats_allreduce": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p), c_double_p]),
         "fbus_stats_allreduce_comm": (C.c_int, [H, C.c_void_p, C.c_void_p, c_double_p]),
         "fbus_synth_streams": (C.c_int, [H, C.POINTER(SynthSpec), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+        "fbus_marker_project": (C.c_int, [H, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32]),
+        "fbus_synth_corners": (C.c_int, [H, C.POINTER(CornerSpec), C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p]),
         "fbus_quat_from_rotmat": (None, [c_double_p, c_double_p]),
         "fbus_measure_fp64_peak": (C.c_int, [H, c_double_p]),
     }
@@ -195,7 +204,7 @@ EXPORTED_SYMBOLS = (
     "fbus_batch", "fbus_stream", "fbus_init_gravity_gyrobias", "fbus_iir_prefilter", "fbus_init_position_quaternion", "fbus_propagate",
     "fbus_reset_state", "fbus_update", "fbus_step_windows", "fbus_refract_solve", "fbus_inair_solve", "fbus_undistort_fisheye", "fbus_solve_to_detections", "fbus_refract_solve_gn", "fbus_marker_pose", "fbus_get_state",
     "fbus_set_state", "fbus_clear_status", "fbus_stats", "fbus_stats_combine", "fbus_stats_allreduce", "fbus_stats_allreduce_comm", "fbus_synth_streams", "fbus_quat_from_rotmat",
-    "fbus_measure_fp64_peak", "fbus_set_noise", "fbus_filter_errors")
+    "fbus_measure_fp64_peak", "fbus_set_noise", "fbus_filter_errors", "fbus_marker_project", "fbus_synth_corners")
 
 
 def config_default() -> FbusConfig:

@@ -1155,6 +1155,71 @@ int fbus_synth_streams(fbus_handle* h, const fbus_synth_spec* spec, double* imu_
     return FBUS_OK;
 }
 
+int fbus_marker_project(fbus_handle* h, const double* pose, size_t n, int32_t underwater, double* corners, int32_t* valid, int32_t mem) {
+    if (!h || !pose || !corners || (underwater != 0 && underwater != 1) || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE))
+        return fail(h, FBUS_E_BADARG, "fbus_marker_project: bad argument");
+    if (n == 0) return FBUS_OK;
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    const double* dp;
+    int rc = stage(h, h->scratch_in, pose, 7 * n, mem, &dp);
+    if (rc) return rc;
+    double* dc = corners;
+    int32_t* dv = valid;
+    if (mem == FBUS_MEM_HOST) {
+        CUDA_TRY(h, h->scratch_out.reserve(16 * n * sizeof(double)));
+        CUDA_TRY(h, h->scratch_aux.reserve(n * sizeof(int32_t)));
+        dc = (double*)h->scratch_out.p;
+        dv = valid ? (int32_t*)h->scratch_aux.p : nullptr;
+    }
+    marker_project_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->k, h->gn, dp, n, n, 1, underwater, dc, dv);
+    CUDA_TRY(h, cudaGetLastError());
+    if (mem == FBUS_MEM_HOST) {
+        CUDA_TRY(h, cudaMemcpyAsync(corners, dc, 16 * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        if (valid) CUDA_TRY(h, cudaMemcpyAsync(valid, dv, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    }
+    return FBUS_OK;
+}
+
+int fbus_synth_corners(fbus_handle* h, const fbus_corner_spec* spec, size_t w0, size_t w1, float* corners, int32_t* ids) {
+    if (!h || !spec || !corners || !ids || !spec->base_pose || !spec->base_id) return fail(h, FBUS_E_BADARG, "fbus_synth_corners: bad argument");
+    const size_t m = spec->max_markers, W = spec->n_frames;
+    if (w0 > w1 || w1 > W || m == 0) return fail(h, FBUS_E_BADARG, "fbus_synth_corners: need w0 <= w1 <= n_frames and max_markers > 0");
+    // Philox counters: the global frame index is one 32-bit word, the slot's streams must stay below 2^32
+    if (W > 0xFFFFFFFFull || m > (0xFFFFFFFFull - CORNER_STREAM0) / CORNER_STREAM_STRIDE)
+        return fail(h, FBUS_E_BADARG, "fbus_synth_corners: n_frames or max_markers too large");
+    if (spec->underwater != 0 && spec->underwater != 1) return fail(h, FBUS_E_BADARG, "fbus_synth_corners: underwater must be 0 or 1");
+    if (!(spec->sigma_corner >= 0.0) || !(spec->sigma_outlier >= 0.0)) return fail(h, FBUS_E_BADARG, "fbus_synth_corners: negative sigma");
+    if (!(spec->p_drop >= 0.0 && spec->p_drop <= 1.0) || !(spec->p_outlier >= 0.0 && spec->p_outlier <= 1.0))
+        return fail(h, FBUS_E_BADARG, "fbus_synth_corners: probability outside [0, 1]");
+    const size_t nws = (w1 - w0) * m, n = nws * h->B;
+    if (n == 0) return FBUS_OK;
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    // the noise-free corners of each (frame, slot) of the range, projected once for all filters
+    CUDA_TRY(h, h->scratch_in.reserve(nws * 7 * sizeof(double)));
+    CUDA_TRY(h, h->scratch_out.reserve(nws * 16 * sizeof(double)));
+    CUDA_TRY(h, h->scratch_aux.reserve(nws * 2 * sizeof(int32_t)));
+    double* dpose = (double*)h->scratch_in.p;
+    double* dbase = (double*)h->scratch_out.p;
+    int32_t* did = (int32_t*)h->scratch_aux.p;
+    int32_t* dvalid = did + nws;
+    CUDA_TRY(h, cudaMemcpyAsync(dpose, spec->base_pose + w0 * m * 7, nws * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(did, spec->base_id + w0 * m, nws * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    marker_project_kernel<<<(unsigned)((nws + 127) / 128), 128, 0, h->stream>>>(h->k, h->gn, dpose, nws, 1, 7, spec->underwater, dbase, dvalid);
+    CUDA_TRY(h, cudaGetLastError());
+    CornerSynthParams sp;
+    memset(&sp, 0, sizeof sp);
+    sp.B = h->B; sp.m = m; sp.n = n; sp.w0 = w0;
+    sp.base = dbase; sp.base_id = did; sp.base_valid = dvalid;
+    sp.corners = corners; sp.ids = ids;
+    sp.s_corner = spec->sigma_corner; sp.p_drop = spec->p_drop; sp.p_out = spec->p_outlier; sp.s_out = spec->sigma_outlier;
+    sp.seed = spec->seed; sp.filter_offset = spec->filter_offset;
+    synth_corners_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(sp);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));  // base arrays staged from caller memory: make reuse safe
+    return FBUS_OK;
+}
+
 int fbus_measure_fp64_peak(fbus_handle* h, double* flops) {
     if (!h || !flops) return fail(h, FBUS_E_BADARG, "fbus_measure_fp64_peak: bad argument");
     CUDA_TRY(h, cudaSetDevice(h->device));

@@ -509,6 +509,84 @@ __global__ void __launch_bounds__(128) synth_kernel(const __grid_constant__ Synt
     }
 }
 
+// ---- forward model and per-filter stereo corner streams (fbus_marker_project, fbus_synth_corners) ----------------------
+// One thread per marker: pose element e of marker i at pose[e * ld_e + i * ld_i] (ld_e = n, ld_i = 1: the [7][n] layout of
+// fbus_marker_project; ld_e = 1, ld_i = 7: the [n][7] rows of fbus_corner_spec.base_pose) -> corners [16][n], valid [n] or null
+__global__ void __launch_bounds__(128) marker_project_kernel(const __grid_constant__ DevConsts k, const __grid_constant__ GnConsts g,
+                                                             const double* __restrict__ pose, size_t n, size_t ld_e, size_t ld_i, int underwater,
+                                                             double* __restrict__ corners, int32_t* __restrict__ valid) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double ps[7], uv[16];
+#pragma unroll
+    for (int e = 0; e < 7; ++e) ps[e] = pose[(size_t)e * ld_e + i * ld_i];
+    const bool ok = project_marker(k, g, underwater, ps, uv);
+#pragma unroll
+    for (int e = 0; e < 16; ++e) corners[(size_t)e * n + i] = uv[e];
+    if (valid) valid[i] = ok ? 1 : 0;
+}
+
+// Philox streams of fbus_synth_corners: slot s draws from streams CORNER_STREAM0 + CORNER_STREAM_STRIDE * s + d, d = 0..7 the
+// white noise (coordinates 2d, 2d+1), 8 the drop / outlier uniforms, 9..16 the outlier normals.  All >= 64: disjoint from
+// synth_kernel's streams 0-2, 16-18 and 32-35, so one seed drives both generators independently.
+constexpr uint32_t CORNER_STREAM0 = 64u, CORNER_STREAM_STRIDE = 32u;
+struct CornerSynthParams {
+    size_t B, m, n;              // n = (w1 - w0) * m * B items, item ((w - w0) * m + slot) * B + b
+    size_t w0;                   // global index of the first frame (the Philox counter uses global frames)
+    const double* base;          // device [16][(w1 - w0) * m]: noise-free corners of each (frame, slot)
+    const int32_t* base_id;      // device [(w1 - w0) * m]: marker id, < 0 = empty slot
+    const int32_t* base_valid;   // device [(w1 - w0) * m]: projection valid
+    float* corners;              // [16][n]
+    int32_t* ids;                // [n]
+    double s_corner, p_drop, p_out, s_out;
+    uint64_t seed, filter_offset;
+};
+__device__ __forceinline__ double uniform53(uint32_t hi, uint32_t lo) {  // [0,1)
+    return (double)((((uint64_t)hi << 32) | lo) >> 11) * (1.0 / 9007199254740992.0);
+}
+__global__ void __launch_bounds__(128) synth_corners_kernel(const __grid_constant__ CornerSynthParams sp) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= sp.n) return;
+    const size_t ws = i / sp.B, b = i % sp.B;  // (frame, slot) of this chunk; filter
+    const uint32_t w = (uint32_t)(sp.w0 + ws / sp.m);
+    const uint32_t st = CORNER_STREAM0 + CORNER_STREAM_STRIDE * (uint32_t)(ws % sp.m);
+    const uint64_t gf = sp.filter_offset + b;
+    const size_t nws = sp.n / sp.B;
+    int32_t id = sp.base_valid[ws] ? sp.base_id[ws] : -1;
+    bool outlier = false;
+    if (id >= 0) {
+        uint32_t r[4];
+        philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), w, st + 8u, (uint32_t)sp.seed, (uint32_t)(sp.seed >> 32), r);
+        if (uniform53(r[0], r[1]) < sp.p_drop) id = -1;
+        else outlier = uniform53(r[2], r[3]) < sp.p_out;
+    }
+    sp.ids[i] = id;
+    if (id < 0) {
+#pragma unroll
+        for (int e = 0; e < 16; ++e) sp.corners[(size_t)e * sp.n + i] = 0.0f;
+        return;
+    }
+    double c[16];
+#pragma unroll
+    for (int d = 0; d < 8; ++d) {
+        double z0, z1;
+        normal2(sp.seed, gf, w, st + (uint32_t)d, &z0, &z1);
+        c[2 * d] = sp.base[(size_t)(2 * d) * nws + ws] + sp.s_corner * z0;
+        c[2 * d + 1] = sp.base[(size_t)(2 * d + 1) * nws + ws] + sp.s_corner * z1;
+    }
+    if (outlier) {
+#pragma unroll
+        for (int d = 0; d < 8; ++d) {
+            double z0, z1;
+            normal2(sp.seed, gf, w, st + 9u + (uint32_t)d, &z0, &z1);
+            c[2 * d] += sp.s_out * z0;
+            c[2 * d + 1] += sp.s_out * z1;
+        }
+    }
+#pragma unroll
+    for (int e = 0; e < 16; ++e) sp.corners[(size_t)e * sp.n + i] = (float)c[e];
+}
+
 // ---- FP64 FMA peak microbenchmark: 8 independent DFMA chains per thread ----------------------------
 __global__ void __launch_bounds__(256) fp64_peak_kernel(double* out, int iters, double seed) {
     double a0 = seed, a1 = seed + 1, a2 = seed + 2, a3 = seed + 3, a4 = seed + 4, a5 = seed + 5, a6 = seed + 6, a7 = seed + 7;

@@ -594,4 +594,47 @@ FBUS_HD void quat_to_rotmat_unit(const double* q, double* R) {
     q2R(qn, R);
 }
 
+// Forward model of one marker (fbus_marker_project): pose[7] = p xyz, q wxyz of corner 0 in the flipped left-camera frame ->
+// uv[16] = left (x,y) of corners 0..3, then right, the input layout of the solves.  Corner geometry and un-flip as in
+// gn_normal_eq; underwater: right camera through R_RL_inv / P_LR and the exact (non-FAST) flat-port projection; in air: the
+// pinhole geometry of VISION::NormalTriangulation, x_R ~ T_LR_air [X_L; 1].  Returns false, with all 16 outputs NaN, when a
+// corner lies at or behind the port (Z <= d_air + d_glass underwater, Z <= 0 in air) in either camera's frame.
+FBUS_HD bool project_marker(const DevConsts& k, const GnConsts& g, int underwater, const double* pose, double* uv) {
+    double Rm[9];
+    quat_to_rotmat_unit(pose + 3, Rm);
+    const double zmin = underwater ? g.d0 + g.d1 : 0.0;
+    bool ok = true;
+    for (int i = 0; i < 4 && ok; ++i) {
+        const double cx = (i == 1 || i == 2) ? g.size : 0.0, cy = (i >= 2) ? g.size : 0.0;
+        const double XL[3] = {-(pose[0] + Rm[0] * cx + Rm[1] * cy), -(pose[1] + Rm[3] * cx + Rm[4] * cy), pose[2] + Rm[6] * cx + Rm[7] * cy};
+        for (int cam = 0; cam < 2; ++cam) {
+            double X[3];
+            if (cam == 0) {
+                X[0] = XL[0]; X[1] = XL[1]; X[2] = XL[2];
+            } else if (underwater) {
+                const double dL[3] = {XL[0] - g.P_LR[0], XL[1] - g.P_LR[1], XL[2] - g.P_LR[2]};
+                mat3_vec(g.R_RL_inv, dL, X);
+            } else {
+                FBUS_UNROLL
+                for (int r = 0; r < 3; ++r)
+                    X[r] = k.T_LR_air[r * 4] * XL[0] + k.T_LR_air[r * 4 + 1] * XL[1] + k.T_LR_air[r * 4 + 2] * XL[2] + k.T_LR_air[r * 4 + 3];
+            }
+            if (!(X[2] > zmin)) { ok = false; break; }  // also catches a non-finite pose
+            double* o = uv + cam * 8 + 2 * i;
+            if (underwater) {
+                double s = 0.0;
+                project_refr<false, false>(g, X, o, nullptr, s);
+            } else {
+                o[0] = X[0] / X[2];
+                o[1] = X[1] / X[2];
+            }
+        }
+    }
+    if (!ok) {
+        FBUS_UNROLL
+        for (int e = 0; e < 16; ++e) uv[e] = (double)NAN;
+    }
+    return ok;
+}
+
 }  // namespace fbus

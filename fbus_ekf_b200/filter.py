@@ -229,6 +229,30 @@ class BatchFilter:
     def SynthStreams(self, spec: capi.SynthSpec, imu_ptr: int, det_id_ptr: int, det_pose_ptr: int, bias_ptr: int | None = None):
         self._ck(self._lib.fbus_synth_streams(self._h, C.byref(spec), imu_ptr, det_id_ptr, det_pose_ptr, bias_ptr))
 
+    def MarkerProject(self, pose, underwater: bool = True, n: int | None = None, corners=None, valid=None,
+                      mem: int = capi.FBUS_MEM_HOST):
+        """Forward model of the stereo front end (fbus_marker_project): marker poses float64 [7][n] (p xyz, q wxyz of corner 0,
+        flipped left-camera frame) -> (corners float64 [16][n], valid int32 [n]) in the input layout of RefractSolve /
+        InAirSolve; an invalid item's corners are NaN.  With mem = FBUS_MEM_DEVICE, pose, corners and valid (or None) are
+        device pointers and n is required."""
+        if mem == capi.FBUS_MEM_HOST:
+            pose = np.ascontiguousarray(pose, dtype=np.float64)
+            assert pose.ndim == 2 and pose.shape[0] == 7, pose.shape
+            n = pose.shape[1]
+            corners = np.empty((16, n))
+            valid = np.empty(n, dtype=np.int32)
+            self._ck(self._lib.fbus_marker_project(self._h, pose.ctypes.data, n, int(underwater), corners.ctypes.data,
+                                                   valid.ctypes.data, mem))
+            return corners, valid
+        self._ck(self._lib.fbus_marker_project(self._h, int(pose), int(n), int(underwater), int(corners),
+                                               int(valid) if valid is not None else None, mem))
+        return corners, valid
+
+    def SynthCorners(self, spec: capi.CornerSpec, w0: int, w1: int, corners_ptr: int, ids_ptr: int):
+        """Per-filter stereo corner streams of frames [w0, w1) (fbus_synth_corners) into DEVICE buffers: corners float32
+        [16][(w1-w0)*m*B], ids int32 [w1-w0][m][B], the input of SolveToDetections"""
+        self._ck(self._lib.fbus_synth_corners(self._h, C.byref(spec), int(w0), int(w1), int(corners_ptr), int(ids_ptr)))
+
     def MeasureFp64Peak(self) -> float:
         v = C.c_double(0.0)
         self._ck(self._lib.fbus_measure_fp64_peak(self._h, C.byref(v)))

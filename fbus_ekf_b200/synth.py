@@ -9,6 +9,8 @@ GPU by fbus_synth_streams (Philox4x32-10).  Nothing here is on the timed path.
   forward_project      flat-port forward projection (air -> glass -> water) of 3-D points into normalised image
                        coordinates (SURVEY A.1-4); inverse of the ray trace of VISION::RefractionTriangulation.
   random_marker_corners  stereo corner observations of randomly posed square markers (config 4 input).
+  base_marker_poses    noise-free pose of every map marker in every frame of a truth trajectory; with make_corner_spec the
+                       input of fbus_synth_corners, which projects them and adds per-filter corner noise on the device.
 """
 from __future__ import annotations
 
@@ -348,3 +350,44 @@ def board_base_corners(cfg: capi.FbusConfig, traj: dict):
         out[8 + 2 * i], out[9 + 2 * i] = uvR[:, 0], uvR[:, 1]
     ids = np.tile(np.arange(m, dtype=np.int32)[None, :], (W, 1))
     return np.ascontiguousarray(out), np.ascontiguousarray(ids), p_all
+
+
+# white noise on the normalised corner coordinates of the logs (2e-4, the level of BASELINE configs[3] and random_marker_corners)
+DEFAULT_CORNER_NOISE = 2e-4
+
+
+def base_marker_poses(cfg: capi.FbusConfig, traj: dict):
+    """noise-free pose of every map marker for every frame of the truth trajectory, as the filter's own measurement model
+    predicts it (the first half of board_base_corners): p = R_IL R^T (P_M - p_true - R P_IL), q = Q_IL * conj(q_true) * Q_M (not
+    normalised; the projection normalises it).  -> (pose float64 [W][m][7], ids int32 [W][m] = the map's marker ids)"""
+    R_IL, Q_IL, P_IL = filter_extrinsics(cfg)
+    m, W = cfg.n_markers, traj["truth_p"].shape[0]
+    pose = np.zeros((W, m, 7))
+    for w in range(W):
+        q = traj["truth_q"][w]
+        R = _q2R(q)
+        for s in range(m):
+            P_M = np.array(cfg.marker_pos[3 * s:3 * s + 3])
+            Q_M = quat_from_rotmat(np.array(cfg.marker_rot[9 * s:9 * s + 9]).reshape(3, 3))
+            pose[w, s, 0:3] = R_IL @ R.T @ (P_M - traj["truth_p"][w] - R @ P_IL)
+            pose[w, s, 3:7] = _qmul(_qmul(Q_IL, _qconj(q)), Q_M)
+    ids = np.tile(np.array(cfg.marker_id[:m], dtype=np.int32)[None, :], (W, 1))
+    return np.ascontiguousarray(pose), np.ascontiguousarray(ids)
+
+
+def make_corner_spec(pose: np.ndarray, ids: np.ndarray, seed: int, filter_offset: int = 0, underwater: bool = True,
+                     sigma_corner: float = DEFAULT_CORNER_NOISE, p_drop: float = 0.0, p_outlier: float = 0.0,
+                     sigma_outlier: float = 0.0) -> capi.CornerSpec:
+    """fbus_corner_spec over base poses [W][m][7] and ids [W][m] (base_marker_poses); the arrays are kept alive by the spec"""
+    pose = np.ascontiguousarray(pose, dtype=np.float64)
+    ids = np.ascontiguousarray(ids, dtype=np.int32)
+    assert pose.ndim == 3 and pose.shape[2] == 7 and ids.shape == pose.shape[:2], (pose.shape, ids.shape)
+    sp = capi.CornerSpec()
+    sp.n_frames, sp.max_markers = pose.shape[0], pose.shape[1]
+    sp.base_pose = capi.dptr(pose)
+    sp.base_id = capi.dptr(ids, capi.c_int32_p)
+    sp.underwater = int(underwater)
+    sp.sigma_corner, sp.p_drop, sp.p_outlier, sp.sigma_outlier = sigma_corner, p_drop, p_outlier, sigma_outlier
+    sp.seed, sp.filter_offset = seed, filter_offset
+    sp._keep = (pose, ids)
+    return sp

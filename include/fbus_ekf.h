@@ -35,7 +35,8 @@ extern "C" {
 #endif
 
 #define FBUS_ABI_VERSION 3 /* 2: fbus_config.imu_g / gn_tol, fbus_imu_stream.format, fbus_iir_prefilter; 3: fbus_stats_allreduce*, FBUS_E_NCCL;
-                              added within 3 (no struct changed): fbus_set_noise, fbus_filter_errors */
+                              added within 3 (no struct changed): fbus_set_noise, fbus_filter_errors, fbus_marker_project,
+                              fbus_synth_corners with the new fbus_corner_spec */
 
 /* error codes */
 #define FBUS_OK 0
@@ -410,6 +411,54 @@ typedef struct fbus_synth_spec {
    [6][B]) receives the drawn b_a, b_g. */
 int fbus_synth_streams(fbus_handle* h, const fbus_synth_spec* spec, double* imu_data, int32_t* det_id,
                        double* det_pose, double* bias_out);
+
+/*
+ * Forward model of the stereo front end (not in the reference; the exact inverse of fbus_refract_solve / fbus_inair_solve):
+ *   pose    [7][n]  double: p xyz, q wxyz of corner 0 in the flipped left-camera frame (the layout the solves write); the
+ *                           quaternion is normalised before use;
+ *   corners [16][n] double: left (x,y) of corners 0..3, then right, normalised coordinates (the solves' input layout);
+ *   valid   [n] int32 or NULL: 1, or 0 when one of the 8 corner points lies at or behind the port in its camera's frame
+ *                           (Z <= d_air + d_glass underwater, Z <= 0 in air); that item's 16 outputs are then NaN.
+ * Corners (0,0,0), (s,0,0), (s,s,0), (0,s,0) of the marker (s = marker_size) are un-flipped into the left camera frame.
+ * underwater = 1: the right camera through the true inverse of R_RL and P_LR, and the flat-port projection air -> glass ->
+ * water solved by Newton iterations to 4.5e-16 relative (the one the Gauss-Newton refinement uses, with its paraxial branch);
+ * underwater = 0: the pinhole geometry of VISION::NormalTriangulation, x_R ~ [R_IR R_IL^T | P_LI - R P_RI] [X_L; 1].
+ * mem applies to all three pointers.
+ */
+int fbus_marker_project(fbus_handle* h, const double* pose, size_t n, int32_t underwater, double* corners, int32_t* valid,
+                        int32_t mem);
+
+typedef struct fbus_corner_spec {
+    size_t n_frames, max_markers;    /* W, m */
+    const double* base_pose;         /* [W][m][7] HOST: noise-free marker pose per slot (flipped left-camera frame) */
+    const int32_t* base_id;          /* [W][m]    HOST: marker id per slot, < 0 = empty */
+    int32_t underwater, reserved;    /* 1: flat-port projection, 0: in air (fbus_marker_project) */
+    double sigma_corner;             /* std of the white noise on every normalised coordinate */
+    double p_drop;                   /* probability that a (frame, slot, filter) detection is missing */
+    double p_outlier, sigma_outlier; /* probability of a gross error; its extra std on all 16 coordinates of the marker */
+    uint64_t seed, filter_offset;    /* as fbus_synth_spec */
+} fbus_corner_spec;
+
+/*
+ * Per-filter stereo corner streams of the marker map, generated ON THE DEVICE for frames [w0, w1) into caller-provided DEVICE
+ * buffers laid out as the input of fbus_solve_to_detections: corners [16][(w1-w0)*m*B] float32 with item
+ * ((w - w0)*m + slot)*B + b, and ids [(w1-w0)][m][B].
+ *   1. The noise-free corners of a (frame, slot) are fbus_marker_project of its base pose, computed once for all filters.
+ *   2. A slot with base id < 0, or whose projection is not valid, gets id -1 and zero corners in every filter.
+ *   3. Otherwise a uniform draw u_drop < p_drop drops the detection (id -1, zero corners).  A second uniform draw
+ *      u_out < p_outlier makes it an outlier: it keeps its id and every coordinate gets an extra sigma_outlier * z' from
+ *      independent normals.
+ *   4. Each coordinate is base + sigma_corner * z (+ sigma_outlier * z'), summed in double and rounded once to float32 (the
+ *      reference holds corners as cv::Point2f).
+ * Randomness: the Philox4x32-10 / Box-Muller generator of fbus_synth_streams, key = seed, counter = (global filter index
+ * filter_offset + b as two words, GLOBAL frame index w, stream 64 + 32*slot + d): d = 0..7 the normals of coordinates 2d and
+ * 2d+1, d = 8 the two uniforms (53 bits each, in [0,1)), d = 9..16 the outlier normals.  These streams are disjoint from those of
+ * fbus_synth_streams, so one seed drives both calls independently; frame ranges split over several calls, and batches split
+ * into shards with filter_offset, give bit-for-bit the output of one call.
+ * FBUS_E_BADARG: NULL outputs or base arrays, w0 > w1, w1 > n_frames, max_markers == 0, a negative sigma, a probability outside
+ * [0, 1], underwater not 0 or 1.  Synchronises (the base arrays are staged from host memory).
+ */
+int fbus_synth_corners(fbus_handle* h, const fbus_corner_spec* spec, size_t w0, size_t w1, float* corners, int32_t* ids);
 
 /* ---- helpers with no device work (usable without a GPU) ----------------------------------- */
 
