@@ -112,44 +112,87 @@ int fail(fbus_handle* h, int code, const std::string& msg) {
             return fail(h, FBUS_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));         \
     } while (0)
 
-// stage a caller array on the device if it lives on the host; returns the device pointer to use
-template <class T>
-int stage_on(fbus_handle* h, DevBuf& buf, const T* src, size_t count, int mem, const T** out, cudaStream_t st) {
-    if (mem == FBUS_MEM_DEVICE) {
-        *out = src;
-        return FBUS_OK;
-    }
-    CUDA_TRY(h, buf.reserve(count * sizeof(T)));
-    CUDA_TRY(h, cudaMemcpyAsync(buf.p, src, count * sizeof(T), cudaMemcpyHostToDevice, st));
-    *out = (const T*)buf.p;
+// Every memory kind a caller passes is checked here, before the call has any effect; the code after the check holds it as `host`.
+int check_mem(fbus_handle* h, int32_t mem, const char* call, bool* host) {
+    if (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE)
+        return fail(h, FBUS_E_BADARG, std::string(call) + ": memory kind must be FBUS_MEM_HOST or FBUS_MEM_DEVICE");
+    *host = mem == FBUS_MEM_HOST;
     return FBUS_OK;
 }
-template <class T>
-int stage(fbus_handle* h, DevBuf& buf, const T* src, size_t count, int mem, const T** out) {
-    return stage_on(h, buf, src, count, mem, out, h->stream);
-}
 
-// IMU samples of either element format: bytes per value, validation, and the (imu, imu32) pointer pair of the kernels
+// IMU samples of either element format: bytes per value and the (imu, imu32) pointer pair of the kernels
 inline size_t imu_elem(const fbus_imu_stream* imu) { return imu->format == FBUS_IMU_F32_SENSOR ? sizeof(float) : sizeof(double); }
-inline bool imu_format_ok(const fbus_imu_stream* imu) { return imu->format == FBUS_IMU_F64_SI || imu->format == FBUS_IMU_F32_SENSOR; }
 inline void set_imu_ptr(const fbus_imu_stream* imu, const void* base, const double** p64, const float** p32) {
     const bool f32 = imu->format == FBUS_IMU_F32_SENSOR;
     *p64 = f32 ? nullptr : (const double*)base;
     *p32 = f32 ? (const float*)base : nullptr;
 }
-// stages values [first, first + count) of the stream's bulk array (count values, not samples) if it lives on the host
-int stage_imu(fbus_handle* h, const fbus_imu_stream* imu, size_t first, size_t count, const void** out) {
-    const size_t es = imu_elem(imu);
-    const char* src = (const char*)imu->data + first * es;
-    if (imu->mem == FBUS_MEM_DEVICE) {
+
+// an IMU stream of which the call reads samples [first, first + count), and their timestamps if need_t
+int check_imu(fbus_handle* h, const fbus_imu_stream* imu, size_t first, size_t count, bool need_t, const char* call, bool* host) {
+    if (!h || !imu || imu->batch != h->B || first > imu->n_samples || count > imu->n_samples - first || !imu->data ||
+        (need_t && !imu->t) || (imu->format != FBUS_IMU_F64_SI && imu->format != FBUS_IMU_F32_SENSOR))
+        return fail(h, FBUS_E_BADARG, std::string(call) + ": bad imu stream");
+    return check_mem(h, imu->mem, call, host);
+}
+
+// detection frames of which the call reads frames [w0, w1)
+int check_det(fbus_handle* h, const fbus_det_frames* det, size_t w0, size_t w1, const char* call, bool* host) {
+    if (!det || det->batch != h->B || w1 > det->n_frames || w0 > w1 || det->max_markers == 0 || !det->t || !det->id || !det->pose)
+        return fail(h, FBUS_E_BADARG, std::string(call) + ": bad detection frames");
+    // the kernel keeps a frame's update slots as a 32-bit mask
+    if ((h->k.flags & FBUS_FLAG_ALL_MARKERS) && det->max_markers > 32)
+        return fail(h, FBUS_E_BADARG, std::string(call) + ": FBUS_FLAG_ALL_MARKERS: max_markers > 32");
+    return check_mem(h, det->mem, call, host);
+}
+
+// A caller's input array on the device: host memory is copied into `buf` on the handle's stream, device memory is used in place.
+template <class T>
+int stage(fbus_handle* h, DevBuf& buf, const T* src, size_t count, bool host, const T** out) {
+    if (!host) {
         *out = src;
         return FBUS_OK;
     }
-    CUDA_TRY(h, h->imu_data.reserve(count * es));
-    CUDA_TRY(h, cudaMemcpyAsync(h->imu_data.p, src, count * es, cudaMemcpyHostToDevice, h->stream));
-    *out = h->imu_data.p;
+    CUDA_TRY(h, buf.reserve(count * sizeof(T)));
+    CUDA_TRY(h, cudaMemcpyAsync(buf.p, src, count * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+    *out = (const T*)buf.p;
     return FBUS_OK;
 }
+// values [first, first + count) of the stream's bulk array (values, not samples) on the device, as the kernels' pointer pair
+int stage_imu(fbus_handle* h, const fbus_imu_stream* imu, bool host, size_t first, size_t count, const double** p64, const float** p32) {
+    const size_t es = imu_elem(imu);
+    const char* d;
+    int rc = stage(h, h->imu_data, (const char*)imu->data + first * es, count * es, host, &d);
+    if (rc == FBUS_OK) set_imu_ptr(imu, d, p64, p32);
+    return rc;
+}
+
+// The outputs of a one-shot call.  Device memory: the kernel writes the caller's arrays.  Host memory: it writes handle
+// scratch, which finish() copies back to every array the caller passed before it waits for the stream once.
+struct Outputs {
+    fbus_handle* h;
+    bool host;
+    int n = 0;
+    struct { void* dst; const void* src; size_t bytes; } copy[3];
+
+    int reserve(DevBuf& buf, size_t bytes) {
+        if (host) CUDA_TRY(h, buf.reserve(bytes));
+        return FBUS_OK;
+    }
+    // the array the kernel writes `count` elements of `dst` to: `dst` itself, or `scratch` (reserved) for host memory
+    template <class T>
+    T* to(T* dst, void* scratch, size_t count) {
+        if (!host) return dst;
+        if (dst) copy[n++] = {dst, scratch, count * sizeof(T)};
+        return (T*)scratch;
+    }
+    int finish() {
+        if (!host) return FBUS_OK;
+        for (int i = 0; i < n; ++i) CUDA_TRY(h, cudaMemcpyAsync(copy[i].dst, copy[i].src, copy[i].bytes, cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        return FBUS_OK;
+    }
+};
 
 // the continuation rule of fbus_step_windows ends here: the next fused call starts with an empty IMU buffer at win_off[w0]
 inline void forget_stream_position(fbus_handle* h) {
@@ -254,29 +297,28 @@ cudaError_t set_window_smem_limits() {
     return e;
 }
 
-int stage_det(fbus_handle* h, const fbus_det_frames* det, size_t w0, size_t w1, WinParams& prm, cudaStream_t big_stream = nullptr) {
-    if (!det || det->batch != h->B || w1 > det->n_frames || w0 > w1 || det->max_markers == 0 || !det->t || !det->id || !det->pose)
-        return fail(h, FBUS_E_BADARG, "bad detection frames");
-    const size_t m = det->max_markers, B = h->B, nw = w1 - w0;
-    if ((h->k.flags & FBUS_FLAG_ALL_MARKERS) && m > 32) return fail(h, FBUS_E_BADARG, "FBUS_FLAG_ALL_MARKERS: max_markers > 32");
-    // timestamps are always host memory; stage only the frames of this call, re-based to index 0
-    const double* dt;
-    int rc = stage(h, h->det_t, det->t + w0, nw, FBUS_MEM_HOST, &dt);
+// fbus_init_position_quaternion (M_INIT), fbus_reset_state (M_RESET) and fbus_update (M_UPDATE): one un-fused step of the
+// window kernel on one frame, staged re-based to index 0
+int step_frame(fbus_handle* h, const fbus_det_frames* det, size_t frame, int32_t mode, size_t n_imu_before, const char* call) {
+    if (!h) return FBUS_E_BADARG;
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    bool host;
+    int rc = check_det(h, det, frame, frame + 1, call, &host);
     if (rc) return rc;
-    const int32_t* did;
-    const double* dpose;
-    cudaStream_t bs = big_stream ? big_stream : h->stream;
-    rc = stage_on(h, h->det_id, det->id + w0 * m * B, nw * m * B, det->mem, &did, bs);
-    if (rc) return rc;
-    rc = stage_on(h, h->det_pose, det->pose + w0 * m * 7 * B, nw * m * 7 * B, det->mem, &dpose, bs);
-    if (rc) return rc;
-    prm.det_t = dt;
-    prm.det_id = did;
-    prm.det_pose = dpose;
+    const size_t m = det->max_markers, B = h->B;
+    WinParams prm;
+    memset(&prm, 0, sizeof prm);
+    // timestamps are always host memory
+    if ((rc = stage(h, h->det_t, det->t + frame, 1, true, &prm.det_t))) return rc;
+    if ((rc = stage(h, h->det_id, det->id + frame * m * B, m * B, host, &prm.det_id))) return rc;
+    if ((rc = stage(h, h->det_pose, det->pose + frame * m * 7 * B, m * 7 * B, host, &prm.det_pose))) return rc;
     prm.m = (int32_t)m;
     prm.w0 = 0;
-    prm.w1 = (uint32_t)nw;
-    return FBUS_OK;
+    prm.w1 = 1;
+    prm.mode = mode;
+    prm.n_imu_before = (uint32_t)n_imu_before;
+    if (mode == M_INIT) forget_stream_position(h);  // the un-fused initialisation stands outside any fused call's IMU buffer
+    return launch_window(h, prm);
 }
 
 }  // namespace
@@ -442,17 +484,15 @@ size_t fbus_batch(const fbus_handle* h) { return h ? h->B : 0; }
 void* fbus_stream(fbus_handle* h) { return h ? (void*)h->stream : nullptr; }
 
 int fbus_init_gravity_gyrobias(fbus_handle* h, const fbus_imu_stream* imu, size_t first, size_t count) {
-    if (!h || !imu || imu->batch != h->B || first + count > imu->n_samples || !imu->data || !imu_format_ok(imu))
-        return fail(h, FBUS_E_BADARG, "bad imu stream");
+    bool host;
+    int rc = check_imu(h, imu, first, count, false, "fbus_init_gravity_gyrobias", &host);
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (count == 0) return FBUS_OK;
     forget_stream_position(h);  // InitializeGravityAndBias clears the IMU buffer (filter.cpp:279)
-    const void* d;
-    int rc = stage_imu(h, imu, first * 6 * h->B, count * 6 * h->B, &d);
-    if (rc) return rc;
     const double* d64;
     const float* d32;
-    set_imu_ptr(imu, d, &d64, &d32);
+    if ((rc = stage_imu(h, imu, host, first * 6 * h->B, count * 6 * h->B, &d64, &d32))) return rc;
     const unsigned grid = (unsigned)((h->B + 127) / 128);
     init_gravity_kernel<<<grid, 128, 0, h->stream>>>(h->d_nom, h->B, d64, d32, h->k.imu_g, 0u, (uint32_t)count);
     CUDA_TRY(h, cudaGetLastError());
@@ -460,61 +500,41 @@ int fbus_init_gravity_gyrobias(fbus_handle* h, const fbus_imu_stream* imu, size_
 }
 
 int fbus_iir_prefilter(fbus_handle* h, const fbus_imu_stream* imu, size_t first, size_t count, double* out, int32_t out_mem) {
-    if (!h || !imu || imu->batch != h->B || first + count > imu->n_samples || !imu->data || !imu_format_ok(imu) || !out ||
-        (out_mem != FBUS_MEM_HOST && out_mem != FBUS_MEM_DEVICE))
-        return fail(h, FBUS_E_BADARG, "fbus_iir_prefilter: bad argument");
+    static const char* const call = "fbus_iir_prefilter";
+    bool host, out_host;
+    int rc = check_imu(h, imu, first, count, false, call, &host);
+    if (rc) return rc;
+    if (!out) return fail(h, FBUS_E_BADARG, "fbus_iir_prefilter: bad argument");
+    if ((rc = check_mem(h, out_mem, call, &out_host))) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (count == 0) return FBUS_OK;
     const size_t n = count * 6 * h->B;
-    const void* d;
-    int rc = stage_imu(h, imu, first * 6 * h->B, n, &d);
-    if (rc) return rc;
     const double* d64;
     const float* d32;
-    set_imu_ptr(imu, d, &d64, &d32);
-    double* dout = out;
-    if (out_mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve(n * sizeof(double)));
-        dout = (double*)h->scratch_out.p;
-    }
+    if ((rc = stage_imu(h, imu, host, first * 6 * h->B, n, &d64, &d32))) return rc;
+    Outputs o{h, out_host};
+    if ((rc = o.reserve(h->scratch_out, n * sizeof(double)))) return rc;
+    double* dout = o.to(out, h->scratch_out.p, n);
     const unsigned grid = (unsigned)((6 * h->B + 127) / 128);
     iir_prefilter_kernel<<<grid, 128, 0, h->stream>>>(d64, d32, h->k.imu_g, h->B, 0u, (uint32_t)count, dout);
     CUDA_TRY(h, cudaGetLastError());
-    if (out_mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(out, dout, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_init_position_quaternion(fbus_handle* h, const fbus_det_frames* det, size_t frame, size_t n_imu_before) {
-    if (!h) return FBUS_E_BADARG;
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    WinParams prm;
-    memset(&prm, 0, sizeof prm);
-    int rc = stage_det(h, det, frame, frame + 1, prm);
-    if (rc) return rc;
-    prm.mode = M_INIT;
-    prm.n_imu_before = (uint32_t)n_imu_before;
-    forget_stream_position(h);  // the un-fused initialisation stands outside any fused call's IMU buffer
-    return launch_window(h, prm);
+    return step_frame(h, det, frame, M_INIT, n_imu_before, "fbus_init_position_quaternion");
 }
 
 int fbus_propagate(fbus_handle* h, const fbus_imu_stream* imu, size_t first, size_t count, double t_end) {
-    if (!h || !imu || imu->batch != h->B || first + count > imu->n_samples || !imu->t || !imu->data || !imu_format_ok(imu))
-        return fail(h, FBUS_E_BADARG, "bad imu stream");
+    bool host;
+    int rc = check_imu(h, imu, first, count, true, "fbus_propagate", &host);
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (count == 0) return FBUS_OK;
     WinParams prm;
     memset(&prm, 0, sizeof prm);
-    const double* dt;
-    const void* dd;
-    int rc = stage(h, h->imu_t, imu->t + first, count, FBUS_MEM_HOST, &dt);
-    if (rc) return rc;
-    rc = stage_imu(h, imu, first * 6 * h->B, count * 6 * h->B, &dd);
-    if (rc) return rc;
-    prm.imu_t = dt;
-    set_imu_ptr(imu, dd, &prm.imu, &prm.imu32);
+    if ((rc = stage(h, h->imu_t, imu->t + first, count, true, &prm.imu_t))) return rc;
+    if ((rc = stage_imu(h, imu, host, first * 6 * h->B, count * 6 * h->B, &prm.imu, &prm.imu32))) return rc;
     prm.mode = M_PROP;
     prm.prop_first = 0;
     prm.prop_count = (uint32_t)count;
@@ -525,25 +545,11 @@ int fbus_propagate(fbus_handle* h, const fbus_imu_stream* imu, size_t first, siz
 }
 
 int fbus_reset_state(fbus_handle* h, const fbus_det_frames* det, size_t frame) {
-    if (!h) return FBUS_E_BADARG;
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    WinParams prm;
-    memset(&prm, 0, sizeof prm);
-    int rc = stage_det(h, det, frame, frame + 1, prm);
-    if (rc) return rc;
-    prm.mode = M_RESET;
-    return launch_window(h, prm);
+    return step_frame(h, det, frame, M_RESET, 0, "fbus_reset_state");
 }
 
 int fbus_update(fbus_handle* h, const fbus_det_frames* det, size_t frame) {
-    if (!h) return FBUS_E_BADARG;
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    WinParams prm;
-    memset(&prm, 0, sizeof prm);
-    int rc = stage_det(h, det, frame, frame + 1, prm);
-    if (rc) return rc;
-    prm.mode = M_UPDATE;
-    return launch_window(h, prm);
+    return step_frame(h, det, frame, M_UPDATE, 0, "fbus_update");
 }
 
 // Fused frames [w0, w1) of a stream.  The kernel indexes the stream with absolute sample / frame numbers (the small host arrays
@@ -552,14 +558,11 @@ int fbus_update(fbus_handle* h, const fbus_det_frames* det, size_t frame) {
 //   host-resident bulk arrays, one launch : samples [win_off[w0], win_off[w1]) and frames [w0, w1) are staged (no continuation)
 //   host-resident, pipelined             : device buffers for the whole range, filled chunk by chunk on the copy stream while the
 //                                          previous chunk is computed; chunks after the first continue (cursor_resume)
-static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const fbus_det_frames* det, const uint32_t* win_off,
-                              size_t w0, size_t w1, double* trace, int32_t trace_mem, bool resume, size_t chunk_frames) {
+static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, bool imu_host, const fbus_det_frames* det, bool det_host,
+                              const uint32_t* win_off, size_t w0, size_t w1, double* trace, bool trace_host, bool resume,
+                              size_t chunk_frames) {
     const size_t B = h->B, nw = w1 - w0, m = det->max_markers;
-    if (det->batch != B || w1 > det->n_frames || m == 0 || !det->t || !det->id || !det->pose) return fail(h, FBUS_E_BADARG, "bad detection frames");
-    // the kernel keeps a frame's update slots as a 32-bit mask
-    if ((h->k.flags & FBUS_FLAG_ALL_MARKERS) && m > 32) return fail(h, FBUS_E_BADARG, "FBUS_FLAG_ALL_MARKERS: max_markers > 32");
     const size_t s0 = win_off[w0], s1 = win_off[w1];
-    const bool imu_host = imu->mem == FBUS_MEM_HOST, det_host = det->mem == FBUS_MEM_HOST;
     WinParams prm;
     memset(&prm, 0, sizeof prm);
     const size_t es = imu_elem(imu);  // bytes per IMU value: double (SI) or float (sensor units)
@@ -600,15 +603,15 @@ static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const 
         dpose = (const double*)(h->pack_dev + o_pose) - w0 * m * 7 * B;
     } else {
         if (s1) {
-            rc = stage(h, h->imu_t, imu->t, s1, FBUS_MEM_HOST, &dt);
+            rc = stage(h, h->imu_t, imu->t, s1, true, &dt);
             if (rc) return rc;
         } else {  // an empty sample range: imu->t may be empty too, the kernel indexes no sample
             CUDA_TRY(h, h->imu_t.reserve(sizeof(double)));
             dt = (const double*)h->imu_t.p;
         }
-        rc = stage(h, h->win_off, win_off, w1 + 1, FBUS_MEM_HOST, &doff);
+        rc = stage(h, h->win_off, win_off, w1 + 1, true, &doff);
         if (rc) return rc;
-        rc = stage(h, h->det_t, det->t, w1, FBUS_MEM_HOST, &ddt);
+        rc = stage(h, h->det_t, det->t, w1, true, &ddt);
         if (rc) return rc;
     }
     if (imu_host && !packed) {
@@ -623,7 +626,7 @@ static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const 
     }
     double* dtrace = nullptr;
     if (trace) {
-        if (trace_mem == FBUS_MEM_DEVICE) dtrace = trace;
+        if (!trace_host) dtrace = trace;
         else {
             CUDA_TRY(h, h->trace.reserve(nw * 17 * B * sizeof(double)));
             dtrace = (double*)h->trace.p;
@@ -668,7 +671,7 @@ static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const 
         rc = launch_window(h, prm);
         if (rc) return rc;
     }
-    if (trace && trace_mem == FBUS_MEM_HOST) {
+    if (trace && trace_host) {
         CUDA_TRY(h, cudaMemcpyAsync(trace, dtrace, nw * 17 * B * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     }
@@ -677,25 +680,32 @@ static int step_windows_range(fbus_handle* h, const fbus_imu_stream* imu, const 
 
 int fbus_step_windows(fbus_handle* h, const fbus_imu_stream* imu, const fbus_det_frames* det, const uint32_t* win_off,
                       size_t w0, size_t w1, double* trace, int32_t trace_mem) {
-    if (!h || !imu || !det || !win_off || imu->batch != h->B || !imu->t || !imu->data || !imu_format_ok(imu))
-        return fail(h, FBUS_E_BADARG, "fbus_step_windows: bad argument");
+    static const char* const call = "fbus_step_windows";
+    bool imu_host, det_host, trace_host;
+    if (!det || !win_off) return fail(h, FBUS_E_BADARG, "fbus_step_windows: bad argument");
+    // samples [0, win_off[w1]): the kernel indexes the stream with absolute sample numbers
+    int rc = check_imu(h, imu, 0, w0 < w1 ? win_off[w1] : 0, true, call, &imu_host);
+    if (rc) return rc;
+    if ((rc = check_mem(h, trace_mem, call, &trace_host))) return rc;
     if (w0 >= w1) return (w0 == w1) ? FBUS_OK : fail(h, FBUS_E_BADARG, "fbus_step_windows: w0 > w1");
     CUDA_TRY(h, cudaSetDevice(h->device));
     for (size_t w = w0; w < w1; ++w)
         if (win_off[w + 1] < win_off[w]) return fail(h, FBUS_E_BADARG, "fbus_step_windows: win_off must be non-decreasing");
-    if (win_off[w1] > imu->n_samples) return fail(h, FBUS_E_BADARG, "fbus_step_windows: win_off beyond the IMU stream");
+    if ((rc = check_det(h, det, w0, w1, call, &det_host))) {  // a bad detection descriptor ends the continuation
+        forget_stream_position(h);
+        return rc;
+    }
     const size_t nw = w1 - w0, B = h->B;
     // Continuation (see the header): the call picks up where the previous one on this handle stopped -- same device-resident
     // IMU array, w0 equal to the previous w1 -- so samples a filter has not consumed yet stay buffered across the two calls.
-    const bool device_streams = imu->mem == FBUS_MEM_DEVICE && det->mem == FBUS_MEM_DEVICE;
+    const bool device_streams = !imu_host && !det_host;
     const bool resume = device_streams && w0 > 0 && w0 == h->last_w1 && imu->data == h->last_imu_data && imu->n_samples == h->last_n_samples;
     // Host-resident streams that are large enough to matter: pipeline the frames in chunks so that the PCIe copy of
     // chunk c+1 runs while chunk c is computed (the state makes one extra HBM round trip per chunk).
     const size_t ch = h->pipeline_frames;
-    const bool host_streams = imu->mem == FBUS_MEM_HOST && det->mem == FBUS_MEM_HOST;
     const size_t bytes = (size_t)(win_off[w1] - win_off[w0]) * 6 * imu_elem(imu) * B;
-    const bool piped = host_streams && ch > 0 && nw >= 2 * ch && bytes >= h->pipeline_min_bytes && h->copy_stream;
-    int rc = step_windows_range(h, imu, det, win_off, w0, w1, trace, trace_mem, resume, piped ? ch : 0);
+    const bool piped = imu_host && det_host && ch > 0 && nw >= 2 * ch && bytes >= h->pipeline_min_bytes && h->copy_stream;
+    rc = step_windows_range(h, imu, imu_host, det, det_host, win_off, w0, w1, trace, trace_host, resume, piped ? ch : 0);
     // a failed call leaves nothing to continue from
     h->last_imu_data = (device_streams && rc == FBUS_OK) ? (const void*)imu->data : nullptr;
     h->last_n_samples = imu->n_samples;
@@ -713,10 +723,14 @@ int fbus_inair_solve(fbus_handle* h, const float* corners, size_t n, double* pos
 }
 static int stereo_solve(fbus_handle* h, const float* corners, size_t n, double* pose, double* corners3d, int32_t* valid, int32_t mem,
                         bool underwater) {
-    if (!h || !corners || !pose) return fail(h, FBUS_E_BADARG, "fbus_refract_solve / fbus_inair_solve: bad argument");
+    const char* const call = underwater ? "fbus_refract_solve" : "fbus_inair_solve";
+    if (!h || !corners || !pose) return fail(h, FBUS_E_BADARG, std::string(call) + ": bad argument");
+    bool host;
+    int rc = check_mem(h, mem, call, &host);
+    if (rc) return rc;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    if (mem != FBUS_MEM_HOST) {
+    if (!host) {
         const unsigned grid = (unsigned)((n + 127) / 128);
         if (underwater) refract_kernel<<<grid, 128, 0, h->stream>>>(h->k, corners, n, n, pose, corners3d, valid);
         else inair_kernel<<<grid, 128, 0, h->stream>>>(h->k, corners, n, n, pose, corners3d, valid);
@@ -766,109 +780,84 @@ int fbus_solve_to_detections(fbus_handle* h, const float* corners, const int32_t
                              int32_t underwater, int32_t gn_iters, int32_t* det_id, double* det_pose, int32_t mem) {
     if (!h || !corners || !marker_ids || !det_id || !det_pose || max_markers == 0 || gn_iters < 0 || gn_iters > 50)
         return fail(h, FBUS_E_BADARG, "fbus_solve_to_detections: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_solve_to_detections", &host);
+    if (rc) return rc;
     const size_t n = n_frames * max_markers * h->B;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const float* dc;
     const int32_t* di;
-    int rc = stage(h, h->scratch_in, corners, 16 * n, mem, &dc);
-    if (rc) return rc;
-    rc = stage(h, h->scratch_aux, marker_ids, n, mem, &di);
-    if (rc) return rc;
-    int32_t* oid = det_id;
-    double* opose = det_pose;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve(7 * n * sizeof(double) + n * sizeof(int32_t)));
-        opose = (double*)h->scratch_out.p;
-        oid = (int32_t*)(opose + 7 * n);
-    }
+    if ((rc = stage(h, h->scratch_in, corners, 16 * n, host, &dc))) return rc;
+    if ((rc = stage(h, h->scratch_aux, marker_ids, n, host, &di))) return rc;
+    Outputs o{h, host};
+    if ((rc = o.reserve(h->scratch_out, 7 * n * sizeof(double) + n * sizeof(int32_t)))) return rc;
+    double* opose = o.to(det_pose, h->scratch_out.p, 7 * n);
+    int32_t* oid = o.to(det_id, (double*)h->scratch_out.p + 7 * n, n);
     solve_to_det_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->k, h->gn, dc, di, n, h->B, underwater, gn_iters, oid, opose);
     CUDA_TRY(h, cudaGetLastError());
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(det_pose, opose, 7 * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaMemcpyAsync(det_id, oid, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_undistort_fisheye(fbus_handle* h, const float* pixels, size_t n, float* normalised, int32_t mem) {
     if (!h || !pixels || !normalised) return fail(h, FBUS_E_BADARG, "fbus_undistort_fisheye: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_undistort_fisheye", &host);
+    if (rc) return rc;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const float* dp;
-    int rc = stage(h, h->scratch_in, pixels, 16 * n, mem, &dp);
-    if (rc) return rc;
-    float* dout = normalised;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve(16 * n * sizeof(float)));
-        dout = (float*)h->scratch_out.p;
-    }
+    if ((rc = stage(h, h->scratch_in, pixels, 16 * n, host, &dp))) return rc;
+    Outputs o{h, host};
+    if ((rc = o.reserve(h->scratch_out, 16 * n * sizeof(float)))) return rc;
+    float* dout = o.to(normalised, h->scratch_out.p, 16 * n);
     undistort_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->k, dp, n, dout);
     CUDA_TRY(h, cudaGetLastError());
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(normalised, dout, 16 * n * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_refract_solve_gn(fbus_handle* h, const void* corners, int32_t corner_dtype, size_t n, int32_t iters, double* pose,
                           double* cost, int32_t* valid, int32_t mem) {
     if (!h || !corners || !pose || iters < 0 || iters > 50 || (corner_dtype != 0 && corner_dtype != 1))
         return fail(h, FBUS_E_BADARG, "fbus_refract_solve_gn: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_refract_solve_gn", &host);
+    if (rc) return rc;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const size_t esz = corner_dtype ? sizeof(double) : sizeof(float);
-    const void* dc = corners;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_in.reserve(16 * n * esz));
-        CUDA_TRY(h, cudaMemcpyAsync(h->scratch_in.p, corners, 16 * n * esz, cudaMemcpyHostToDevice, h->stream));
-        dc = h->scratch_in.p;
-    }
-    double* dpose = pose;
-    double* dcost = cost;
-    int32_t* dvalid = valid;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve((7 + 1) * n * sizeof(double)));
-        CUDA_TRY(h, h->scratch_aux.reserve(n * sizeof(int32_t)));
-        dpose = (double*)h->scratch_out.p;
-        dcost = dpose + 7 * n;
-        dvalid = (int32_t*)h->scratch_aux.p;
-    }
+    const char* dc;
+    if ((rc = stage(h, h->scratch_in, (const char*)corners, 16 * n * esz, host, &dc))) return rc;
+    Outputs o{h, host};
+    if ((rc = o.reserve(h->scratch_out, (7 + 1) * n * sizeof(double)))) return rc;
+    if ((rc = o.reserve(h->scratch_aux, n * sizeof(int32_t)))) return rc;
+    // for host memory the kernel writes cost and valid to scratch even when the caller does not want them
+    double* dpose = o.to(pose, h->scratch_out.p, 7 * n);
+    double* dcost = o.to(cost, (double*)h->scratch_out.p + 7 * n, n);
+    int32_t* dvalid = o.to(valid, h->scratch_aux.p, n);
     const unsigned grid = (unsigned)((n + 127) / 128);
     if (corner_dtype) refract_gn_kernel<double><<<grid, 128, 0, h->stream>>>(h->k, h->gn, (const double*)dc, n, iters, dpose, dcost, dvalid);
     else refract_gn_kernel<float><<<grid, 128, 0, h->stream>>>(h->k, h->gn, (const float*)dc, n, iters, dpose, dcost, dvalid);
     CUDA_TRY(h, cudaGetLastError());
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(pose, dpose, 7 * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        if (cost) CUDA_TRY(h, cudaMemcpyAsync(cost, dcost, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        if (valid) CUDA_TRY(h, cudaMemcpyAsync(valid, dvalid, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_marker_pose(fbus_handle* h, const double* corners3d, size_t n, double* pose, int32_t mem) {
     if (!h || !corners3d || !pose) return fail(h, FBUS_E_BADARG, "fbus_marker_pose: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_marker_pose", &host);
+    if (rc) return rc;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const double* dc;
-    int rc = stage(h, h->scratch_in, corners3d, 12 * n, mem, &dc);
-    if (rc) return rc;
-    double* dpose = pose;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve(7 * n * sizeof(double)));
-        dpose = (double*)h->scratch_out.p;
-    }
+    if ((rc = stage(h, h->scratch_in, corners3d, 12 * n, host, &dc))) return rc;
+    Outputs o{h, host};
+    if ((rc = o.reserve(h->scratch_out, 7 * n * sizeof(double)))) return rc;
+    double* dpose = o.to(pose, h->scratch_out.p, 7 * n);
     const unsigned grid = (unsigned)((n + 127) / 128);
     marker_pose_kernel<<<grid, 128, 0, h->stream>>>(h->k, dc, n, dpose);
     CUDA_TRY(h, cudaGetLastError());
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(pose, dpose, 7 * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_get_state(fbus_handle* h, fbus_state_soa* out) {
@@ -939,14 +928,15 @@ int fbus_stats_combine(const double* parts, size_t n_parts, double* out) {
 
 int fbus_stats(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem, double* out_host, double* out_dev) {
     if (!h || !truth_p || !truth_q) return fail(h, FBUS_E_BADARG, "fbus_stats: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_stats", &host);
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const size_t B = h->B;
     const double* tp;
     const double* tq;
-    int rc = stage(h, h->scratch_in, truth_p, 3 * B, mem, &tp);
-    if (rc) return rc;
-    rc = stage(h, h->scratch_out, truth_q, 4 * B, mem, &tq);
-    if (rc) return rc;
+    if ((rc = stage(h, h->scratch_in, truth_p, 3 * B, host, &tp))) return rc;
+    if ((rc = stage(h, h->scratch_out, truth_q, 4 * B, host, &tq))) return rc;
     const int grid = (int)((B + STATS_BS - 1) / STATS_BS);
     CUDA_TRY(h, h->stats_partial.reserve((size_t)grid * 8 * sizeof(double)));
     CUDA_TRY(h, h->stats_out.reserve(FBUS_NSTATS * sizeof(double)));
@@ -963,7 +953,10 @@ int fbus_stats(fbus_handle* h, const double* truth_p, const double* truth_q, int
 }
 
 int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem) {
-    if (!h || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE)) return fail(h, FBUS_E_BADARG, "fbus_set_noise: bad argument");
+    if (!h) return fail(h, FBUS_E_BADARG, "fbus_set_noise: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_set_noise", &host);
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (!noise) {  // back to the config's values and the default kernels; the buffer is kept for a later call
         h->noise_on = false;
@@ -976,36 +969,30 @@ int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem) {
     const size_t bytes = (size_t)FBUS_NOISE_FIELDS * h->B * sizeof(double);
     CUDA_TRY(h, h->noise.reserve(bytes));  // allocated on the first call (the size is fixed by the batch)
     // stream-ordered: kernels enqueued before this call still read the previous values
-    CUDA_TRY(h, cudaMemcpyAsync(h->noise.p, noise, bytes, mem == FBUS_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
-                                h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->noise.p, noise, bytes, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
     h->noise_on = true;
     return FBUS_OK;
 }
 
 int fbus_filter_errors(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem, double* out, int32_t out_mem) {
-    if (!h || !truth_p || !truth_q || !out || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE) ||
-        (out_mem != FBUS_MEM_HOST && out_mem != FBUS_MEM_DEVICE))
-        return fail(h, FBUS_E_BADARG, "fbus_filter_errors: bad argument");
+    static const char* const call = "fbus_filter_errors";
+    if (!h || !truth_p || !truth_q || !out) return fail(h, FBUS_E_BADARG, "fbus_filter_errors: bad argument");
+    bool host, out_host;
+    int rc = check_mem(h, mem, call, &host);
+    if (rc == FBUS_OK) rc = check_mem(h, out_mem, call, &out_host);
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const size_t B = h->B;
     const double* tp;
     const double* tq;
-    int rc = stage(h, h->scratch_in, truth_p, 3 * B, mem, &tp);
-    if (rc) return rc;
-    rc = stage(h, h->scratch_out, truth_q, 4 * B, mem, &tq);
-    if (rc) return rc;
-    double* dout = out;
-    if (out_mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->errors.reserve(4 * B * sizeof(double)));
-        dout = (double*)h->errors.p;
-    }
+    if ((rc = stage(h, h->scratch_in, truth_p, 3 * B, host, &tp))) return rc;
+    if ((rc = stage(h, h->scratch_out, truth_q, 4 * B, host, &tq))) return rc;
+    Outputs o{h, out_host};
+    if ((rc = o.reserve(h->errors, 4 * B * sizeof(double)))) return rc;
+    double* dout = o.to(out, h->errors.p, 4 * B);
     filter_errors_kernel<<<(unsigned)((B + STATS_BS - 1) / STATS_BS), STATS_BS, 0, h->stream>>>(h->d_nom, h->d_P, B, tp, tq, dout);
     CUDA_TRY(h, cudaGetLastError());
-    if (out_mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(out, dout, 4 * B * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 // ---- NCCL, loaded at run time: the library itself has no link-time dependency on it ------------------------------------
@@ -1138,9 +1125,9 @@ int fbus_synth_streams(fbus_handle* h, const fbus_synth_spec* spec, double* imu_
     memset(&sp, 0, sizeof sp);
     const double* bi;
     const double* bp;
-    int rc = stage(h, h->scratch_in, spec->base_imu, spec->n_samples * 6, FBUS_MEM_HOST, &bi);
+    int rc = stage(h, h->scratch_in, spec->base_imu, spec->n_samples * 6, true, &bi);
     if (rc) return rc;
-    rc = stage(h, h->scratch_out, spec->base_pose, spec->n_frames * 7, FBUS_MEM_HOST, &bp);
+    rc = stage(h, h->scratch_out, spec->base_pose, spec->n_frames * 7, true, &bp);
     if (rc) return rc;
     sp.B = h->B; sp.N = spec->n_samples; sp.W = spec->n_frames;
     sp.base_imu = bi; sp.base_pose = bp;
@@ -1156,29 +1143,22 @@ int fbus_synth_streams(fbus_handle* h, const fbus_synth_spec* spec, double* imu_
 }
 
 int fbus_marker_project(fbus_handle* h, const double* pose, size_t n, int32_t underwater, double* corners, int32_t* valid, int32_t mem) {
-    if (!h || !pose || !corners || (underwater != 0 && underwater != 1) || (mem != FBUS_MEM_HOST && mem != FBUS_MEM_DEVICE))
-        return fail(h, FBUS_E_BADARG, "fbus_marker_project: bad argument");
+    if (!h || !pose || !corners || (underwater != 0 && underwater != 1)) return fail(h, FBUS_E_BADARG, "fbus_marker_project: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_marker_project", &host);
+    if (rc) return rc;
     if (n == 0) return FBUS_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
     const double* dp;
-    int rc = stage(h, h->scratch_in, pose, 7 * n, mem, &dp);
-    if (rc) return rc;
-    double* dc = corners;
-    int32_t* dv = valid;
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, h->scratch_out.reserve(16 * n * sizeof(double)));
-        CUDA_TRY(h, h->scratch_aux.reserve(n * sizeof(int32_t)));
-        dc = (double*)h->scratch_out.p;
-        dv = valid ? (int32_t*)h->scratch_aux.p : nullptr;
-    }
+    if ((rc = stage(h, h->scratch_in, pose, 7 * n, host, &dp))) return rc;
+    Outputs o{h, host};
+    if ((rc = o.reserve(h->scratch_out, 16 * n * sizeof(double)))) return rc;
+    if ((rc = o.reserve(h->scratch_aux, n * sizeof(int32_t)))) return rc;
+    double* dc = o.to(corners, h->scratch_out.p, 16 * n);
+    int32_t* dv = valid ? o.to(valid, h->scratch_aux.p, n) : nullptr;
     marker_project_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->k, h->gn, dp, n, n, 1, underwater, dc, dv);
     CUDA_TRY(h, cudaGetLastError());
-    if (mem == FBUS_MEM_HOST) {
-        CUDA_TRY(h, cudaMemcpyAsync(corners, dc, 16 * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        if (valid) CUDA_TRY(h, cudaMemcpyAsync(valid, dv, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    return FBUS_OK;
+    return o.finish();
 }
 
 int fbus_synth_corners(fbus_handle* h, const fbus_corner_spec* spec, size_t w0, size_t w1, float* corners, int32_t* ids) {

@@ -46,7 +46,8 @@ extern "C" {
 #define FBUS_E_STATE (-4)
 #define FBUS_E_NCCL (-5) /* NCCL missing (libnccl.so.2 could not be loaded) or an NCCL call failed */
 
-/* where a caller-owned data pointer lives */
+/* where a caller-owned data pointer lives (the mem / out_mem / trace_mem arguments and the mem fields of fbus_imu_stream and
+   fbus_det_frames); a call given any other value returns FBUS_E_BADARG without any effect */
 #define FBUS_MEM_HOST 0
 #define FBUS_MEM_DEVICE 1
 
