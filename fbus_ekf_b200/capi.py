@@ -23,6 +23,7 @@ FBUS_IMU_F32_SENSOR = 1  # float, g and deg/s (the IMSEE SDK's ImuData; converte
 # per-filter status bits (fbus_state_soa.status)
 FBUS_ST_INIT_FAILED, FBUS_ST_RESET_SKIPPED, FBUS_ST_RESET_DONE, FBUS_ST_UPDATE_SKIPPED = 0x1, 0x2, 0x4, 0x8
 FBUS_ST_NONFINITE, FBUS_ST_NO_DETECTION, FBUS_ST_MARKER_REJECTED = 0x10, 0x20, 0x40
+FBUS_ST_UPDATE_REJECTED = 0x80  # rejected by the innovation gate (fbus_set_gate)
 FBUS_FLAG_JOSEPH = 0x1
 FBUS_FLAG_MATLAB = 0x2
 FBUS_FLAG_ALL_MARKERS = 0x4  # every known marker of a frame updates the filter in turn (include/fbus_ekf.h)
@@ -180,6 +181,8 @@ def lib() -> C.CDLL:
         "fbus_stats_combine": (C.c_int, [c_double_p, C.c_size_t, c_double_p]),
         "fbus_set_noise": (C.c_int, [H, C.c_void_p, C.c_int32]),
         "fbus_filter_errors": (C.c_int, [H, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]),
+        "fbus_set_gate": (C.c_int, [H, C.c_void_p, C.c_int32]),
+        "fbus_rejected_updates": (C.c_int, [H, C.c_void_p, C.c_int32]),
         "fbus_stats_allreduce": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p), c_double_p]),
         "fbus_stats_allreduce_comm": (C.c_int, [H, C.c_void_p, C.c_void_p, c_double_p]),
         "fbus_synth_streams": (C.c_int, [H, C.POINTER(SynthSpec), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -204,7 +207,8 @@ EXPORTED_SYMBOLS = (
     "fbus_batch", "fbus_stream", "fbus_init_gravity_gyrobias", "fbus_iir_prefilter", "fbus_init_position_quaternion", "fbus_propagate",
     "fbus_reset_state", "fbus_update", "fbus_step_windows", "fbus_refract_solve", "fbus_inair_solve", "fbus_undistort_fisheye", "fbus_solve_to_detections", "fbus_refract_solve_gn", "fbus_marker_pose", "fbus_get_state",
     "fbus_set_state", "fbus_clear_status", "fbus_stats", "fbus_stats_combine", "fbus_stats_allreduce", "fbus_stats_allreduce_comm", "fbus_synth_streams", "fbus_quat_from_rotmat",
-    "fbus_measure_fp64_peak", "fbus_set_noise", "fbus_filter_errors", "fbus_marker_project", "fbus_synth_corners")
+    "fbus_measure_fp64_peak", "fbus_set_noise", "fbus_filter_errors", "fbus_marker_project", "fbus_synth_corners",
+    "fbus_set_gate", "fbus_rejected_updates")
 
 
 def config_default() -> FbusConfig:

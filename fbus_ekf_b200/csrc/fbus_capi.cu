@@ -86,6 +86,10 @@ struct fbus_handle {
     bool noise_on = false;    // the window kernels read `noise` instead of the config's values
     bool noise_smem_set = false;  // shared-memory limits of the NOISE instantiations set (on the first fbus_set_noise)
     DevBuf errors;            // [4][B] device result of fbus_filter_errors for a host output
+    DevBuf gate, gate_rej;    // [B] thresholds of fbus_set_gate, [B] int32 counts of rejected updates
+    bool gate_on = false;     // the window launches go to the gated instantiations of the first-generation lane kernel
+    bool gate_set = false;    // fbus_set_gate was called with an array: the counts exist
+    bool gate_smem_set = false;  // shared-memory limits of the GATE instantiations set (on the first fbus_set_gate)
     // second staging set + copy stream: host-resident streams are copied chunk c+1 while chunk c is computed
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
@@ -203,7 +207,9 @@ inline void forget_stream_position(fbus_handle* h) {
 
 // NOISE: the instantiations that take every filter's noise values from h->noise (fbus_set_noise); the others get a null
 // pointer they never read
-template <bool NOISE>
+// GATE: the innovation gate (fbus_set_gate): the gated first-generation lanes-per-filter kernel at any batch size; the lane
+// kernel's other instantiations get null pointers they never read
+template <bool NOISE, bool GATE>
 int launch_window_t(fbus_handle* h, WinParams& prm) {
     prm.nom = h->d_nom;
     prm.P = h->d_P;
@@ -218,17 +224,31 @@ int launch_window_t(fbus_handle* h, WinParams& prm) {
     const unsigned grid = (unsigned)((h->B + WIN_BS - 1) / WIN_BS);
     const bool jo = (h->k.flags & FBUS_FLAG_JOSEPH) != 0, f32 = prm.imu32 != nullptr;
     const double* const nz = NOISE ? (const double*)h->noise.p : nullptr;
-    if (h->k.flags & FBUS_FLAG_ALL_MARKERS) {  // every marker of a frame: the first-generation lanes-per-filter kernel at any batch size
+    const GateBufs gt{GATE ? (const double*)h->gate.p : nullptr, GATE ? (int32_t*)h->gate_rej.p : nullptr};
+    if (GATE) {  // (fbus_set_gate refuses a MATLAB-semantics handle)
+        const unsigned g32 = (unsigned)((h->B + 31) / 32);
+        if (h->k.flags & FBUS_FLAG_ALL_MARKERS) {
+            if (f32) {
+                if (jo) ekf_window_lane_kernel<true, true, false, NOISE, true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+                else ekf_window_lane_kernel<false, true, false, NOISE, true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+            } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE, true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+            else ekf_window_lane_kernel<false, false, false, NOISE, true, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        } else if (f32) {
+            if (jo) ekf_window_lane_kernel<true, true, false, NOISE, false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+            else ekf_window_lane_kernel<false, true, false, NOISE, false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE, false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        else ekf_window_lane_kernel<false, false, false, NOISE, false, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+    } else if (h->k.flags & FBUS_FLAG_ALL_MARKERS) {  // every marker of a frame: the first-generation lanes-per-filter kernel at any batch size
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
         if (f32) {
-            if (jo) ekf_window_lane_kernel<true, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-            else ekf_window_lane_kernel<false, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-        else ekf_window_lane_kernel<false, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+            if (jo) ekf_window_lane_kernel<true, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+            else ekf_window_lane_kernel<false, true, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        else ekf_window_lane_kernel<false, false, false, NOISE, true><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
     } else if (h->k.flags & FBUS_FLAG_MATLAB) {  // MATLAB-semantics mode: the lanes-per-filter kernel at any batch size
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
-        if (f32) ekf_window_lane_kernel<false, true, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-        else ekf_window_lane_kernel<false, false, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+        if (f32) ekf_window_lane_kernel<false, true, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        else ekf_window_lane_kernel<false, false, true, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
     } else if (h->lane_batch && h->lane_gen == 2) {
         prm.lane_fpc = h->lane_fpc;
         const unsigned g32 = (unsigned)((h->B + h->lane_fpc - 1) / h->lane_fpc);
@@ -240,10 +260,10 @@ int launch_window_t(fbus_handle* h, WinParams& prm) {
     } else if (h->lane_batch) {
         const unsigned g32 = (unsigned)((h->B + 31) / 32);
         if (f32) {
-            if (jo) ekf_window_lane_kernel<true, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-            else ekf_window_lane_kernel<false, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
-        else ekf_window_lane_kernel<false, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz);
+            if (jo) ekf_window_lane_kernel<true, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+            else ekf_window_lane_kernel<false, true, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        } else if (jo) ekf_window_lane_kernel<true, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
+        else ekf_window_lane_kernel<false, false, false, NOISE><<<g32, LANE_NT, LANE_SMEM, h->stream>>>(prm, h->k, nz, gt);
     } else if (h->small_batch) {
         // fewer 128-filter CTAs than SMs (e.g. BASELINE configs[2], 4 096 filters): 32-filter CTAs (one covariance + one
         // nominal warp) spread the batch over four times as many SMs
@@ -262,7 +282,10 @@ int launch_window_t(fbus_handle* h, WinParams& prm) {
     CUDA_TRY(h, cudaGetLastError());
     return FBUS_OK;
 }
-int launch_window(fbus_handle* h, WinParams& prm) { return h->noise_on ? launch_window_t<true>(h, prm) : launch_window_t<false>(h, prm); }
+int launch_window(fbus_handle* h, WinParams& prm) {
+    if (h->gate_on) return h->noise_on ? launch_window_t<true, true>(h, prm) : launch_window_t<false, true>(h, prm);
+    return h->noise_on ? launch_window_t<true, false>(h, prm) : launch_window_t<false, false>(h, prm);
+}
 
 // the largest dynamic shared memory of every window kernel of one NOISE flavour (the default is 48 KB)
 template <bool NOISE>
@@ -294,6 +317,30 @@ cudaError_t set_window_smem_limits() {
     set((const void*)ekf_window_lane2_kernel<true, false, NOISE>, LANE2_SMEM);
     set((const void*)ekf_window_lane2_kernel<false, true, NOISE>, LANE2_SMEM);
     set((const void*)ekf_window_lane2_kernel<true, true, NOISE>, LANE2_SMEM);
+    return e;
+}
+// the same for the GATE instantiations of the first-generation lane kernel (both NOISE flavours)
+cudaError_t set_gate_smem_limits() {
+    cudaError_t e = cudaSuccess;
+    auto set = [&](const void* fn) {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LANE_SMEM);
+    };
+    set((const void*)ekf_window_lane_kernel<false, false, false, false, false, true>);
+    set((const void*)ekf_window_lane_kernel<true, false, false, false, false, true>);
+    set((const void*)ekf_window_lane_kernel<false, true, false, false, false, true>);
+    set((const void*)ekf_window_lane_kernel<true, true, false, false, false, true>);
+    set((const void*)ekf_window_lane_kernel<false, false, false, false, true, true>);
+    set((const void*)ekf_window_lane_kernel<true, false, false, false, true, true>);
+    set((const void*)ekf_window_lane_kernel<false, true, false, false, true, true>);
+    set((const void*)ekf_window_lane_kernel<true, true, false, false, true, true>);
+    set((const void*)ekf_window_lane_kernel<false, false, false, true, false, true>);
+    set((const void*)ekf_window_lane_kernel<true, false, false, true, false, true>);
+    set((const void*)ekf_window_lane_kernel<false, true, false, true, false, true>);
+    set((const void*)ekf_window_lane_kernel<true, true, false, true, false, true>);
+    set((const void*)ekf_window_lane_kernel<false, false, false, true, true, true>);
+    set((const void*)ekf_window_lane_kernel<true, false, false, true, true, true>);
+    set((const void*)ekf_window_lane_kernel<false, true, false, true, true, true>);
+    set((const void*)ekf_window_lane_kernel<true, true, false, true, true, true>);
     return e;
 }
 
@@ -467,7 +514,8 @@ int fbus_destroy(fbus_handle* h) {
         if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]);
     }
     DevBuf* bufs[] = {&h->imu_t, &h->det_t, &h->win_off, &h->imu_data, &h->det_id, &h->det_pose, &h->trace,
-                      &h->scratch_in, &h->scratch_out, &h->scratch_aux, &h->stats_partial, &h->stats_out, &h->noise, &h->errors};
+                      &h->scratch_in, &h->scratch_out, &h->scratch_aux, &h->stats_partial, &h->stats_out, &h->noise, &h->errors,
+                      &h->gate, &h->gate_rej};
     for (DevBuf* b : bufs) b->release();
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -972,6 +1020,46 @@ int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem) {
     CUDA_TRY(h, cudaMemcpyAsync(h->noise.p, noise, bytes, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
     h->noise_on = true;
     return FBUS_OK;
+}
+
+int fbus_set_gate(fbus_handle* h, const double* gate, int32_t mem) {
+    if (!h) return fail(h, FBUS_E_BADARG, "fbus_set_gate: bad argument");
+    bool host;
+    int rc = check_mem(h, mem, "fbus_set_gate", &host);
+    if (rc) return rc;
+    if (h->k.flags & FBUS_FLAG_MATLAB) return fail(h, FBUS_E_BADARG, "fbus_set_gate: not available with FBUS_FLAG_MATLAB");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    if (!gate) {  // back to the default kernels; thresholds and counts are kept
+        h->gate_on = false;
+        return FBUS_OK;
+    }
+    if (!h->gate_smem_set) {  // the GATE instantiations are prepared when first needed: creation only touches the default ones
+        CUDA_TRY(h, set_gate_smem_limits());
+        h->gate_smem_set = true;
+    }
+    const size_t B = h->B;
+    CUDA_TRY(h, h->gate.reserve(B * sizeof(double)));  // allocated on the first call (the size is fixed by the batch)
+    CUDA_TRY(h, h->gate_rej.reserve(B * sizeof(int32_t)));
+    // stream-ordered: kernels enqueued before this call still read the previous thresholds and add to the previous counts
+    CUDA_TRY(h, cudaMemcpyAsync(h->gate.p, gate, B * sizeof(double), host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(h->gate_rej.p, 0, B * sizeof(int32_t), h->stream));
+    h->gate_on = true;
+    h->gate_set = true;
+    return FBUS_OK;
+}
+
+int fbus_rejected_updates(fbus_handle* h, int32_t* out, int32_t out_mem) {
+    if (!h || !out) return fail(h, FBUS_E_BADARG, "fbus_rejected_updates: bad argument");
+    bool out_host;
+    int rc = check_mem(h, out_mem, "fbus_rejected_updates", &out_host);
+    if (rc) return rc;
+    if (!h->gate_set) return fail(h, FBUS_E_STATE, "fbus_rejected_updates: no gate was set on this handle");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    Outputs o{h, out_host};
+    int32_t* dst = o.to(out, h->gate_rej.p, h->B);  // host: finish() copies the counts themselves back
+    if (dst != h->gate_rej.p)
+        CUDA_TRY(h, cudaMemcpyAsync(dst, h->gate_rej.p, h->B * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
+    return o.finish();
 }
 
 int fbus_filter_errors(fbus_handle* h, const double* truth_p, const double* truth_q, int32_t mem, double* out, int32_t out_mem) {

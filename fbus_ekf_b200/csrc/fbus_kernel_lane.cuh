@@ -140,7 +140,8 @@ __device__ __forceinline__ void lane_apply_Fu1(double* x, const double* A, const
 // NOISE: q0, q1 come from this filter's row of the [6][B] buffer `noise` (fbus_set_noise) instead of k.Qd
 // ALL: FBUS_FLAG_ALL_MARKERS -- after the first update of a frame, further update rounds follow until no filter of the CTA
 // requests one (nominal_role posts one marker per filter and round)
-template <bool JOSEPH, bool NOISE = false, bool ALL = false>
+// GATE: the innovation gate -- after (c) a filter's request is read again, the nominal lane has withdrawn a rejected one
+template <bool JOSEPH, bool NOISE = false, bool ALL = false, bool GATE = false>
 __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh, int32_t (*sflag)[32],
                                               int cw, int lane, const double* noise = nullptr) {
     constexpr int NT = LANE_NT;
@@ -232,12 +233,14 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
             }
             cta_bar<NT>();  // (p) P6 published
             cta_bar<NT>();  // (c) the nominal warp has posted Lc and y
+            bool upd = req;  // GATE: not withdrawn by the gate
+            if constexpr (GATE) upd = req && sflag[2][f] != 0;
             // own columns of the factor Z with (I-KH)P = P - Z^T Z, dx = Z^T y:
             //   default  Z = X G   (7 x 18), X = L^-1 Hs, y = z = L^-1 r      (S = L L^T)
             //   Joseph   Z = Lc^T G (6 x 18), Lc Lc^T = C_J, y = Lc^-1 u       (update_prologue)
             constexpr int NZ = JOSEPH ? 6 : 7;
             double z0[NZ], z1[NZ];
-            if (req) {
+            if (upd) {
                 if constexpr (JOSEPH) {
                     double Cm[21];
 #pragma unroll
@@ -281,7 +284,7 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
                 X[(size_t)(LX_DX + 9 + l) * 32] = d1;
             }
             __syncwarp();  // the filter's Z columns are in its scratch
-            if (req) {
+            if (upd) {
 #pragma unroll
                 for (int r = 0; r < 18; ++r) {  // P -= Z^T Z on both columns (exactly symmetric: the same products in the same order on both sides)
                     double v0 = c0[r], v1 = c1[r];
@@ -312,20 +315,24 @@ __device__ __forceinline__ void lane_cov_role(const WinParams& prm, const DevCon
 // NOISE: every filter has its own noise values, `noise` is the [6][B] buffer of fbus_set_noise (the other instantiations never
 // read the parameter)
 // ALL: FBUS_FLAG_ALL_MARKERS, every known marker of a frame updates the filter in turn (include/fbus_ekf.h)
-template <bool JOSEPH, bool IMU32, bool MATLAB = false, bool NOISE = false, bool ALL = false>
+// GATE: the innovation gate of fbus_set_gate, thresholds and counts in `gate` (the other instantiations never read the parameter)
+template <bool JOSEPH, bool IMU32, bool MATLAB = false, bool NOISE = false, bool ALL = false, bool GATE = false>
 __global__ void __launch_bounds__(LANE_NT, 1) ekf_window_lane_kernel(const __grid_constant__ WinParams prm, const __grid_constant__ DevConsts k,
-                                                                     const double* __restrict__ noise) {
+                                                                     const double* __restrict__ noise, const GateBufs gate) {
     extern __shared__ double smem[];
     __shared__ SplitShared sh;
     __shared__ int32_t sflag[3][32];
     const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (wi < 11) {
-        if constexpr (NOISE) lane_cov_role<JOSEPH, true, ALL>(prm, k, smem, sh, sflag, wi, lane, noise);
-        else lane_cov_role<JOSEPH, false, ALL>(prm, k, smem, sh, sflag, wi, lane);
+        if constexpr (NOISE) lane_cov_role<JOSEPH, true, ALL, GATE>(prm, k, smem, sh, sflag, wi, lane, noise);
+        else lane_cov_role<JOSEPH, false, ALL, GATE>(prm, k, smem, sh, sflag, wi, lane);
     } else {
         const size_t b0 = (size_t)blockIdx.x * 32 + lane;
         const bool live = b0 < prm.B;
-        if constexpr (NOISE)
+        if constexpr (GATE)
+            nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, NOISE, ALL, true>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1,
+                                                                                          live, nullptr, nullptr, nullptr, noise, gate);
+        else if constexpr (NOISE)
             nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, true, ALL>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live,
                                                                                    nullptr, nullptr, nullptr, noise);
         else nominal_role<32, false, IMU32, true, JOSEPH, MATLAB, false, false, ALL>(prm, k, smem, sh, sflag, lane, live ? b0 : prm.B - 1, live);

@@ -611,6 +611,21 @@ struct P6View {
     }
 };
 
+// The innovation gate of fbus_set_gate (first-generation lanes-per-filter kernel): per-filter thresholds [B] and the per-filter
+// counts of rejected updates [B]
+struct GateBufs {
+    const double* thr;
+    int32_t* rejected;
+};
+// NIS = r^T S^-1 r = |z|^2 of z = L^-1 r (S = L L^T); the update is rejected iff thr > 0 and not NIS <= thr, so a non-finite NIS
+// is rejected and a threshold <= 0 or NaN gates nothing
+__device__ __forceinline__ bool gate_rejects(const double* z, double thr) {
+    double nis = z[0] * z[0];
+#pragma unroll
+    for (int i = 1; i < 7; ++i) nis += z[i] * z[i];
+    return thr > 0.0 && !(nis <= thr);
+}
+
 // LANE = true: the role runs inside the lanes-per-filter kernel (fbus_kernel_lane.cuh): every barrier is CTA-wide, invalid ring
 // records need no neutral content, and the update is split differently -- this warp (one lane per filter) runs the
 // state-only prologue (predicted measurement, Hs, S, the gain factors) from the published P6 and the error-state
@@ -619,11 +634,15 @@ struct P6View {
 // ALL (first-generation LANE only): FBUS_FLAG_ALL_MARKERS -- the update hand-off (r) (p) (c) (d) repeats, one marker per filter and
 // round (the planned one, then pl.extra in slot order), each at the state the previous injection left, until a round in which no
 // filter of the CTA posts a request; the next frame's plan is made in the first round only
+// GATE (first-generation LANE only): the innovation gate of fbus_set_gate -- after the prologue every update whose NIS fails the
+// filter's threshold is withdrawn (sflag[2] cleared before (c), which the covariance lanes re-read) and not injected; the
+// filter's count of rejections is kept in a register and written once at the end
 template <int BSF, bool TM, bool IMU32 = false, bool LANE = false, bool JOSEPH = false, bool MATLAB = false, bool LANE2 = false,
-          bool NOISE = false, bool ALL = false>
+          bool NOISE = false, bool ALL = false, bool GATE = false>
 __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevConsts& k, double* smem, SplitShared& sh,
                                              int32_t (*sflag)[BSF], int fl, size_t b, bool live, Lane2Shared* l2 = nullptr,
-                                             const MarkerTable* tab_smem = nullptr, double* ring2 = nullptr, const double* noise = nullptr) {
+                                             const MarkerTable* tab_smem = nullptr, double* ring2 = nullptr, const double* noise = nullptr,
+                                             GateBufs gt = GateBufs{nullptr, nullptr}) {
     const MarkerTable* const tab = tab_smem ? tab_smem : prm.tab;  // the second-generation lane kernel keeps a copy in shared memory
     constexpr int NT = LANE ? LANE_NT : 2 * BSF, NW = BSF / 32;
     static_assert(!LANE || BSF == 32, "the lanes-per-filter kernel has 32 filters per CTA");
@@ -631,6 +650,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
     static_assert(!LANE2 || (LANE && !MATLAB), "the second-generation lanes-per-filter kernel has the C++ semantics only");
     static_assert(!NOISE || LANE, "the warp-specialised kernel applies R in its covariance role");
     static_assert(!ALL || (LANE && !LANE2 && !MATLAB), "the all-markers mode runs on the first-generation lanes-per-filter kernel, C++ semantics");
+    static_assert(!GATE || (LANE && !LANE2 && !MATLAB), "the innovation gate runs on the first-generation lanes-per-filter kernel, C++ semantics");
     constexpr int REC = LANE ? LX_REC : 22;  // doubles per ring slot
     constexpr int LXS = LANE2 ? L2_SHIFT : 0;  // shift of the exchange sections behind the ring
     const size_t B = prm.B;
@@ -658,6 +678,12 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
     int prev_id = prm.prev_id[b];
     int inited = prm.init[b];
     int status = prm.status[b];
+    double gthr = 0.0;    // GATE: this filter's threshold
+    int32_t n_rej = 0;    // GATE: its count of rejected updates
+    if constexpr (GATE) {
+        gthr = gt.thr[b];
+        n_rej = gt.rejected[b];
+    }
     uint32_t cursor = fused ? (prm.cursor_resume ? prm.cursor_io[b] : prm.win_off[prm.w0]) : 0u;
     // first IMU sample of the NEXT window, prefetched while this warp waits for the covariance warp's update
     uint32_t pf_i = 0xffffffffu;
@@ -919,6 +945,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
         nx.do_prop = nx.apply_init = nx.apply_reset = false;
         nx.req = 0;
         for (uint32_t round = 0;; ++round) {
+        bool rej = false;  // GATE: this round's update of this filter failed the gate
         // ---- F4 ObservationUpdate (filter.cpp:622-739): post the request (into the ring slot the covariance warp is
         //      not reading), the covariance warp does the algebra ------------------------------------------------
         if (req && !LANE) {
@@ -947,15 +974,19 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
                 if (req) {
                     const MarkerConst mkc = tab->mk[req - 1];
                     if constexpr (JOSEPH) {  // 6-row factor Lc of the Joseph-form C_J and y = Lc^-1 u
-                        double Cm[21], yv[6];
+                        double Cm[21], yv[6], zg[7];
                         if constexpr (NOISE) {
                             const MeasNoise r{noise[4 * B + b], noise[5 * B + b]};
                             update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, r, mkc, pl.y, pl.y + 3, Cm,
-                                                                    yv, X + (size_t)(LXS + LX_SCR) * BSF);
+                                                                    yv, X + (size_t)(LXS + LX_SCR) * BSF, GATE ? zg : nullptr);
+                        } else if constexpr (GATE) {
+                            update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, k, mkc, pl.y, pl.y + 3, Cm,
+                                                                    yv, X + (size_t)(LXS + LX_SCR) * BSF, zg);
                         } else {
                             update_prologue<BSF, BSF, true, P6View>(P6View{X + (size_t)(LXS + LX_P6) * BSF}, n, k, mkc, pl.y, pl.y + 3, Cm, yv,
                                                                     X + (size_t)(LXS + LX_SCR) * BSF);
                         }
+                        if constexpr (GATE) rej = gate_rejects(zg, gthr);
 #pragma unroll
                         for (int c = 0; c < 21; ++c) X[(size_t)(LXS + LX_CM + c) * BSF] = Cm[c];
 #pragma unroll
@@ -974,6 +1005,12 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
                         }
 #pragma unroll
                         for (int c = 0; c < 7; ++c) X[(size_t)(LXS + LX_Y + c) * BSF] = zv[c];
+                        if constexpr (GATE) rej = gate_rejects(zv, gthr);
+                    }
+                    if (GATE && rej) {  // withdrawn: the covariance lanes re-read the request after (c)
+                        sflag[2][fl] = 0;
+                        status |= FBUS_ST_UPDATE_REJECTED;
+                        ++n_rej;
                     }
                 }
                 L2T(LANE2 && fl == 0, 0, 8);
@@ -994,7 +1031,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
         if (any) {
             sbar(wq);  // (d) results posted
             L2T(LANE2 && fl == 0, 0, 20);
-            if (req) {
+            if (req && !rej) {
                 if constexpr (LANE) {
                     double dx[18];
 #pragma unroll
@@ -1071,6 +1108,7 @@ __device__ __forceinline__ void nominal_role(const WinParams& prm, const DevCons
     prm.init[b] = inited;
     if (fused) prm.cursor_io[b] = cursor;
     prm.status[b] = status;
+    if constexpr (GATE) gt.rejected[b] = n_rej;
     if (MATLAB) prm.nom[(size_t)F_TIMG * B + b] = t_img;
 }
 

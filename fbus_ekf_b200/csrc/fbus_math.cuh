@@ -1167,14 +1167,19 @@ FBUS_HD void update_prologue_sx(const CV P, const KR& k, const UpdHs& hh, double
 // Outputs Cm = lower-packed Cholesky factor Lc of C = Hs^T S^-1 Hs and y = Lc^-1 u (u = Hs^T S^-1 r), so that
 //   (I-KH)P = P - Z^T Z with Z = Lc^T G, and dx = K r = Z^T y.
 // kr: where R comes from (DevConsts or MeasNoise, see MeasNoise)
+// zo (optional): receives z = L^-1 r (7 doubles), whose squared norm is the update's NIS r^T S^-1 r (the innovation gate)
 template <int S, int XS, bool JOSEPH = false, class CV = Cov<S>, class KR = DevConsts>
 FBUS_HD void update_prologue(const CV P, const Nominal& n, const DevConsts& k, const KR& kr, const MarkerConst& mk, const double* yP,
-                             const double* yQ, double* Cm, double* y, double* scr) {
+                             const double* yQ, double* Cm, double* y, double* scr, double* zo = nullptr) {
     double L[28], Li[7], z[7];
     {
         UpdHs hh;
         update_hs(n, k, mk, yP, yQ, hh);
         update_prologue_sx<S, XS, CV>(P, kr, hh, L, Li, z, scr);
+    }
+    if (zo) {
+        FBUS_UNROLL
+        for (int i = 0; i < 7; ++i) zo[i] = z[i];
     }
 #define FBUS_L(i, j) L[(i) * ((i) + 1) / 2 + (j)]
 #define FBUS_X(i) scr[(i) * XS]

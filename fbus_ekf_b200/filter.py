@@ -207,6 +207,31 @@ class BatchFilter:
         else:
             self._ck(self._lib.fbus_set_noise(self._h, int(noise), mem))
 
+    def SetGate(self, gate=None, mem: int = capi.FBUS_MEM_HOST):
+        """Innovation gate (fbus_set_gate): float64 [B] numpy array of per-filter NIS thresholds (<= 0: no gate for that filter),
+        or a device pointer (mem = FBUS_MEM_DEVICE) to such an array.  Resets the rejection counts.  None turns the gate off."""
+        if gate is None:
+            self._ck(self._lib.fbus_set_gate(self._h, None, mem))
+            return
+        if mem == capi.FBUS_MEM_HOST:
+            assert isinstance(gate, np.ndarray) and gate.dtype == np.float64 and gate.flags["C_CONTIGUOUS"], "float64 C-contiguous array"
+            assert gate.shape == (self.batch,), gate.shape
+            self._ck(self._lib.fbus_set_gate(self._h, gate.ctypes.data, mem))
+        else:
+            self._ck(self._lib.fbus_set_gate(self._h, int(gate), mem))
+
+    def RejectedUpdates(self, out=None, out_mem: int = capi.FBUS_MEM_HOST):
+        """Updates rejected per filter since the last SetGate with an array (fbus_rejected_updates) -> int32 [B]: a new numpy
+        array, the given numpy array, or the given device pointer (out_mem = FBUS_MEM_DEVICE)."""
+        if out_mem == capi.FBUS_MEM_HOST:
+            if out is None:
+                out = np.empty(self.batch, dtype=np.int32)
+            assert out.dtype == np.int32 and out.flags["C_CONTIGUOUS"] and out.shape == (self.batch,)
+            self._ck(self._lib.fbus_rejected_updates(self._h, out.ctypes.data, out_mem))
+        else:
+            self._ck(self._lib.fbus_rejected_updates(self._h, int(out), out_mem))
+        return out
+
     def FilterErrors(self, truth_p, truth_q, mem: int = capi.FBUS_MEM_HOST, out=None, out_mem: int = capi.FBUS_MEM_HOST):
         """Per-filter error terms (fbus_filter_errors) -> [4][B]: |p - p_true|^2, |dtheta|^2, NEES (6 dof), finite flag.
         truth_p [3][B], truth_q [4][B] float64 numpy arrays (or device pointers with mem = FBUS_MEM_DEVICE).  Output: a new

@@ -25,6 +25,10 @@ BASELINE configs[3] (synth.board_config) seen from 1 m.  The IMU streams still c
 generated one evaluation chunk at a time, so only the chunk's corners are resident.  These rows also carry detections,
 corner_noise, p_drop, p_outlier, sigma_outlier, gn_iters, all_markers, board and n_markers.
 
+Innovation gate (--set gate_chi2=v1,v2,...): one more grid dimension, the NIS threshold of fbus_set_gate (<= 0: no gate).  Every
+filter gets its setting's threshold (same setting-major layout as the noise values), in both detection modes.  Only with
+gate_chi2 in --set do the rows carry gate_chi2 and rejected_per_run (mean count of rejected updates per run at the end).
+
 Validated range: pos_n_cov and quat_n_cov >= 1e-8.  There every kernel form's (position, attitude) covariance block, and so the
 NEES, is within 1e-9 relative of a 50-digit evaluation (DESIGN.md, "Numerical envelope of the update").  Smaller measurement noise
 runs, but the double-precision update loses digits to cancellation: at 1e-12 the NEES is good to about 1e-7.
@@ -44,6 +48,8 @@ from . import capi
 CHI2_6_95 = 12.591587243743977  # 95 % quantile of the chi-square distribution with 6 degrees of freedom
 MAX_BATCH = 1 << 20
 FRAC_KEY = "frac_nees6_le_12.59"
+GATE_KEY = "gate_chi2"  # the innovation gate's threshold, a grid dimension beside the noise values
+SET_NAMES = capi.NOISE_FIELDS + (GATE_KEY,)
 
 
 def parse_sets(items) -> list[tuple[str, list[float]]]:
@@ -54,8 +60,8 @@ def parse_sets(items) -> list[tuple[str, list[float]]]:
         name = name.strip()
         if not sep or not vals.strip():
             raise ValueError(f"--set {it!r}: expected name=v1,v2,...")
-        if name not in capi.NOISE_FIELDS:
-            raise ValueError(f"--set {it!r}: unknown parameter {name!r} (one of {', '.join(capi.NOISE_FIELDS)})")
+        if name not in SET_NAMES:
+            raise ValueError(f"--set {it!r}: unknown parameter {name!r} (one of {', '.join(SET_NAMES)})")
         if name in seen:
             raise ValueError(f"--set {it!r}: {name} given twice")
         seen.add(name)
@@ -64,7 +70,8 @@ def parse_sets(items) -> list[tuple[str, list[float]]]:
 
 
 def expand_grid(sets, base: dict) -> list[dict]:
-    """Cartesian product of the --set lists over the base values (dict of all six NOISE_FIELDS); the last list varies fastest"""
+    """Cartesian product of the --set lists over the base values (dict of all six NOISE_FIELDS); the last list varies fastest.
+    A setting has gate_chi2 only when it is in `sets`."""
     names = [n for n, _ in sets]
     grid = []
     for combo in itertools.product(*[v for _, v in sets]):
@@ -83,6 +90,18 @@ def noise_array(settings: list[dict], runs: int) -> np.ndarray:
     """[6][len(settings) * runs] fbus_set_noise array, setting-major"""
     col = np.array([[s[n] for n in capi.NOISE_FIELDS] for s in settings], dtype=np.float64).T  # [6][S]
     return np.ascontiguousarray(np.repeat(col, runs, axis=1))
+
+
+def gate_array(settings: list[dict], runs: int) -> np.ndarray | None:
+    """[len(settings) * runs] fbus_set_gate array, setting-major; None when the settings have no gate_chi2"""
+    if GATE_KEY not in settings[0]:
+        return None
+    return np.ascontiguousarray(np.repeat(np.array([s[GATE_KEY] for s in settings], dtype=np.float64), runs))
+
+
+def _rejected_per_run(f, n_set: int, runs: int) -> np.ndarray:
+    """mean count of rejected updates per run, per setting"""
+    return f.RejectedUpdates().reshape(n_set, runs).mean(axis=1)
 
 
 def bytes_per_filter(n_samples: int, n_frames: int, n_markers: int = 1, chunk_frames: int = 0) -> int:
@@ -153,6 +172,9 @@ def run_sweep(sets, runs: int, duration: float, eval_every: float = 1.0, seed: i
         f.SynthStreams(synth.make_synth_spec(traj, seed=seed, filter_offset=s0 * runs, **(data_noise or {})), imu_d.data_ptr(),
                        id_d.data_ptr(), pose_d.data_ptr())
         f.SetNoise(noise_array(grid[s0:s0 + ns], runs))
+        gate = gate_array(grid[s0:s0 + ns], runs)
+        if gate is not None:
+            f.SetGate(gate)
         imu = capi.make_imu_stream(traj["t_imu"], imu_d.data_ptr(), B, capi.FBUS_MEM_DEVICE)
         det = capi.make_det_frames(traj["t_frames"], id_d.data_ptr(), pose_d.data_ptr(), B, 1, capi.FBUS_MEM_DEVICE)
         err = torch.empty((4, B), dtype=torch.float64, device=dev)
@@ -172,14 +194,16 @@ def run_sweep(sets, runs: int, duration: float, eval_every: float = 1.0, seed: i
                 reds.append(_reduce(err, ns, runs))
                 w0 = w1
             red = torch.stack(reds).cpu().numpy()  # [eval][5][S]
+        rej = _rejected_per_run(f, ns, runs) if gate is not None else None
         f.close()
         del imu_d, id_d, pose_d, err
-        rows += _rows(grid[s0:s0 + ns], runs, red, [float(traj["t_frames"][w - 1]) for w in ends])
+        rows += _rows(grid[s0:s0 + ns], runs, red, [float(traj["t_frames"][w - 1]) for w in ends], rej)
     return rows
 
 
-def _rows(settings, runs: int, red, t_eval) -> list[dict]:
-    """one JSON row per setting from the per-evaluation reductions red [eval][5][S] of _reduce"""
+def _rows(settings, runs: int, red, t_eval, rejected=None) -> list[dict]:
+    """one JSON row per setting from the per-evaluation reductions red [eval][5][S] of _reduce (and, with a gate, the mean
+    rejection counts per run [S])"""
     rows = []
     for j, setting in enumerate(settings):
         row = dict(setting)
@@ -190,6 +214,8 @@ def _rows(settings, runs: int, red, t_eval) -> list[dict]:
         row["nees6_mean"] = [float(v) for v in red[:, 2, j]]
         row[FRAC_KEY] = float(red[-1, 3, j])
         row["n_nonfinite"] = int(red[-1, 4, j])
+        if rejected is not None:
+            row["rejected_per_run"] = float(rejected[j])
         rows.append(row)
     return rows
 
@@ -260,6 +286,9 @@ def _run_sweep_corners(sets, runs, duration, eval_every, seed, device, data_nois
         c_d = torch.empty((16, cmax * m * B), dtype=torch.float32, device=dev)
         cid_d = torch.empty((cmax, m, B), dtype=torch.int32, device=dev)
         f.SetNoise(noise_array(grid[s0:s0 + ns], runs))
+        gate = gate_array(grid[s0:s0 + ns], runs)
+        if gate is not None:
+            f.SetGate(gate)
         imu = capi.make_imu_stream(traj["t_imu"], imu_d.data_ptr(), B, capi.FBUS_MEM_DEVICE)
         det = capi.make_det_frames(traj["t_frames"], id_d.data_ptr(), pose_d.data_ptr(), B, m, capi.FBUS_MEM_DEVICE)
         err = torch.empty((4, B), dtype=torch.float64, device=dev)
@@ -279,9 +308,10 @@ def _run_sweep_corners(sets, runs, duration, eval_every, seed, device, data_nois
                 f.Synchronize()
                 reds.append(_reduce(err, ns, runs))
             red = torch.stack(reds).cpu().numpy()  # [eval][5][S]
+        rej = _rejected_per_run(f, ns, runs) if gate is not None else None
         f.close()
         del imu_d, id_d, pose_d, c_d, cid_d, err
-        for row in _rows(grid[s0:s0 + ns], runs, red, [float(traj["t_frames"][w1 - 1]) for _, w1 in chunks]):
+        for row in _rows(grid[s0:s0 + ns], runs, red, [float(traj["t_frames"][w1 - 1]) for _, w1 in chunks], rej):
             row.update(detections="corners", corner_noise=corner_noise, p_drop=p_drop, p_outlier=p_outlier, sigma_outlier=sigma_outlier,
                        gn_iters=gn_iters, all_markers=all_markers, board=board, n_markers=m)
             rows.append(row)
@@ -304,7 +334,8 @@ def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="python -m fbus_ekf_b200.sweep", description=__doc__.split("\n\n")[0],
                                  formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--set", action="append", default=[], metavar="NAME=V1,V2,...",
-                    help=f"values of one noise parameter ({', '.join(capi.NOISE_FIELDS)}); repeat for a grid")
+                    help=f"values of one noise parameter ({', '.join(capi.NOISE_FIELDS)}) or of the innovation gate's NIS threshold "
+                         f"({GATE_KEY}, <= 0: no gate); repeat for a grid")
     ap.add_argument("--runs", type=int, default=4096, help="Monte-Carlo runs per setting (default 4096)")
     ap.add_argument("--duration", type=float, default=5.0, help="seconds of synthetic stream (default 5)")
     ap.add_argument("--eval-every", type=float, default=1.0, help="seconds between evaluations (default 1)")

@@ -36,7 +36,8 @@ extern "C" {
 
 #define FBUS_ABI_VERSION 3 /* 2: fbus_config.imu_g / gn_tol, fbus_imu_stream.format, fbus_iir_prefilter; 3: fbus_stats_allreduce*, FBUS_E_NCCL;
                               added within 3 (no struct changed): fbus_set_noise, fbus_filter_errors, fbus_marker_project,
-                              fbus_synth_corners with the new fbus_corner_spec */
+                              fbus_synth_corners with the new fbus_corner_spec, fbus_set_gate, fbus_rejected_updates,
+                              FBUS_ST_UPDATE_REJECTED */
 
 /* error codes */
 #define FBUS_OK 0
@@ -75,6 +76,7 @@ extern "C" {
 #define FBUS_ST_NONFINITE 0x10       /* a state entry became NaN/Inf */
 #define FBUS_ST_NO_DETECTION 0x20    /* empty detection list for this filter/frame */
 #define FBUS_ST_MARKER_REJECTED 0x40 /* refractive solve: a corner beyond makrer_dect_dist_thres */
+#define FBUS_ST_UPDATE_REJECTED 0x80 /* an update was rejected by the innovation gate (fbus_set_gate) */
 
 /* flags in fbus_config.flags */
 #define FBUS_FLAG_JOSEPH 0x1 /* opt-in Joseph-form covariance update (north_star); default is the
@@ -344,6 +346,36 @@ int fbus_iir_prefilter(fbus_handle* h, const fbus_imu_stream* in, size_t first, 
    fbus_config's.  noise = NULL returns the handle to the config's values.  State, status and the continuation rule of
    fbus_step_windows are untouched: a call between two continued calls takes effect from the next call on. */
 int fbus_set_noise(fbus_handle* h, const double* noise, int32_t mem);
+
+/* ---- innovation gate (chi-square test of every measurement update) --------------------------- */
+
+/* gate[B] doubles (mem as given) or NULL.  Copied into a handle-owned device buffer, like fbus_set_noise.
+    1. Every 7-row measurement update -- the reference's update in the fused path of fbus_step_windows and in fbus_update, and
+       each further update under FBUS_FLAG_ALL_MARKERS -- forms the normalised innovation squared NIS = r^T S^-1 r: r is the
+       7-row residual after the quaternion sign choice, S = H P H^T + R at that update's own linearisation state, R the config's
+       value or, under fbus_set_noise, the filter's own.
+    2. With g = gate[b] the update of filter b is rejected iff g > 0 && !(NIS <= g): a non-finite NIS is rejected, and g <= 0 or
+       NaN means no gate for that filter.
+    3. A rejected update leaves the nominal state and the covariance bit-for-bit unchanged, sets FBUS_ST_UPDATE_REJECTED and adds
+       1 to the filter's count (fbus_rejected_updates).
+    4. Marker selection comes before the gate and is unchanged: prev_marker_id is updated as always.
+    5. Not gated and unchanged: init, reset, the vision-only pose (pv, qv), trace rows, the other status bits and the
+       continuation rule of fbus_step_windows.
+    6. Under FBUS_FLAG_ALL_MARKERS each update of the sequence is gated on its own; a rejected chosen marker does not stop the
+       further slots.
+    7. Combines with FBUS_FLAG_JOSEPH, FBUS_FLAG_ALL_MARKERS, fbus_set_noise and both IMU element formats.  On a FBUS_FLAG_MATLAB
+       handle the call returns FBUS_E_BADARG.  gate = NULL turns the gate off (the window kernels are the default ones again;
+       the counts stay readable).  A call between two continued fbus_step_windows calls takes effect from the next call on.
+    Thresholds: the quaternion rows carry about 3 degrees of freedom plus a second-order component along hQ, so the NIS of a
+    consistent filter lies between chi-square with 6 and with 7 degrees of freedom:
+                     0.95    0.99    0.999
+        chi2(6)     12.59   16.81   22.46
+        chi2(7)     14.07   18.48   24.32
+    Runs on the first-generation lanes-per-filter window kernel at any batch size while a gate is set. */
+int fbus_set_gate(fbus_handle* h, const double* gate, int32_t mem);
+/* out[B] int32 (out_mem as given): updates rejected per filter since the last fbus_set_gate with a non-NULL array.
+   Returns FBUS_E_STATE if the gate was never set on this handle; synchronises for a HOST output. */
+int fbus_rejected_updates(fbus_handle* h, int32_t* out, int32_t out_mem);
 
 /* ---- state access ------------------------------------------------------------------------- */
 
